@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the LORB-SLAM hot path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 The default line carries all three BASELINE metrics: the keyframe-pair sweep is the top-level
 record (descriptor-pairs/s); `ba_batched` (config 4: 512 windows split over the ranks) and
@@ -27,6 +27,18 @@ filter), exact same result as the reference's BFMatcher path.
 Other workloads (`--workload ba_batched | ba_large | ba_local | bf | proj`) put
 another BASELINE config under the same contract; their short versions are also
 reported in `extra` of the default line.
+
+`--steps` sets the timed steps of the sweep and of both BA legs; the short `extra`
+measurements keep their own fixed repetition counts.
+
+`--dump-outputs DIR` writes, after the timed steps, what rank 0's last timed step of
+every workload that ran handed back to its caller, as DIR/<name>.npy (integers as
+float64): on several GPUs that is rank 0's block, window slice and point shard only.
+An array above its share of 64 MB is cut to a fixed, seeded sample of its rows.  The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.  The sweep outputs are exact.  The BA outputs compare
+to a tolerance: their partial sums are accumulated with atomics in no fixed order,
+and the forced attempts past convergence accept or reject on that rounding noise,
+so the trust-region radius and step counts of the BA summaries may differ.
 """
 import argparse
 import json
@@ -187,6 +199,35 @@ def _events(ctx, local):
     return st, torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
 
 
+OUTPUTS = {}  # name -> what rank 0's last timed step returned (see --dump-outputs)
+DUMP_BYTES = 64 * 10 ** 6
+BA_SUMMARY_FIELDS = ("initial_cost", "final_cost", "final_radius", "final_gradient_max_norm", "iterations",
+                     "num_successful_steps", "num_unsuccessful_steps", "termination")
+
+
+def _ba_summary_rows(sums):
+    return np.array([[s[k] for k in BA_SUMMARY_FIELDS] for s in sums], np.float64)
+
+
+def write_outputs(out_dir):
+    """OUTPUTS as out_dir/<name>.npy: float32 stays float32, everything else becomes float64.  Smallest
+    first, every array gets an even share of what is left of DUMP_BYTES (what a small one does not use
+    goes to the larger ones); an array above its share keeps a fixed, seeded sample of its rows (in row
+    order)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {name: np.ascontiguousarray(a, np.float32 if a.dtype == np.float32 else np.float64)
+              for name, a in OUTPUTS.items()}
+    left = DUMP_BYTES
+    for k, name in enumerate(sorted(arrays, key=lambda n: arrays[n].nbytes)):
+        a = arrays[name]
+        share = left // (len(arrays) - k) - 1024  # room for the .npy header
+        if a.nbytes > share:
+            rows = np.random.default_rng(0).choice(len(a), share // (a.nbytes // len(a)), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes + 1024
+
+
 # ----------------------------------------------------------------------- sweep
 def _block_pairs():
     a, b = np.triu_indices(BLOCK_KF, k=1)
@@ -288,7 +329,9 @@ def run_sweep(args, rank, world, local):
     clocks = sampler.stop() if rank == 0 else None
     ms_max = _max_over_ranks(ms, world, local)
     step_ms = ms / args.steps
-    kept_dev = ctx.sweep_plan_download()[0]
+    kept_dev, matches_dev, min_dist_dev = ctx.sweep_plan_download()
+    if rank == 0:
+        OUTPUTS.update(sweep_kept=kept_dev, sweep_matches=matches_dev, sweep_min_dist=min_dist_dev)
     # the dominant kernel alone (the tensor form adds a small finalize kernel per step)
     kernel_ms = step_ms
     if tensor and rank == 0:
@@ -430,6 +473,7 @@ def run_full_sweep(args, rank, world, local, bank):
     if rank == 0:
         from oracle import ref
         allk = dev.cpu().numpy()
+        OUTPUTS["full_sweep_kept"] = allk
         rng = np.random.default_rng(7)
         pa = rng.integers(0, N_KF, 64).astype(np.int32)
         pb = ((pa + rng.integers(BLOCK_KF, N_KF - BLOCK_KF, 64)) % N_KF).astype(np.int32)  # other blocks
@@ -639,13 +683,13 @@ def cpu_baseline_ba_large(pb, iters=2):
                       % (s["iterations"], pb["C"], pb["P"], pb["O"])}
 
 
-def run_ba_batched(args, rank, world, local, steps=None, want_cpu=True):
+def run_ba_batched(args, rank, world, local, want_cpu=True):
     """BASELINE config 4: `--windows-total` (512) independent 10-keyframe windows split in contiguous
     slices over the ranks (strong scaling: the batch is fixed), every window its own LM loop."""
     import torch
     from lorb_slam_b200 import capi, sharding, synth
     _rank_host_threads(world)  # an earlier oracle leg may have taken every core for rank 0
-    steps = steps or args.steps
+    steps = args.steps
     warmup = max(3, min(args.warmup, 3))
     ctx = capi.Context(local)
     total = args.windows_total
@@ -680,6 +724,9 @@ def run_ba_batched(args, rank, world, local, steps=None, want_cpu=True):
     clocks = sampler.stop() if rank == 0 else None
     dt_max = _max_over_ranks(dt, world, local)
     cams_res, pts_res = prob.download()
+    if rank == 0:
+        OUTPUTS.update(ba_batched_cams=cams_res, ba_batched_points=pts_res,
+                       ba_batched_summaries=_ba_summary_rows(sums))
     # parity run: the same windows under Ceres' default tolerances (the timed runs force all 10
     # attempts, and attempts past convergence accept or reject on rounding noise, which makes their
     # end point a coin toss at the 1e-7 level -- not a fair thing to compare bit-for-tolerance)
@@ -756,14 +803,14 @@ def run_ba_batched(args, rank, world, local, steps=None, want_cpu=True):
     return res
 
 
-def run_ba_large(args, rank, world, local, steps=None, want_cpu=True):
+def run_ba_large(args, rank, world, local, want_cpu=True):
     """BASELINE config 5 BA: 200 keyframes / 200k points / 1.5M observations, points sharded over the
     ranks, reduced camera system all-reduced over NCCL every LM attempt.  Strong scaling."""
     import torch
     _rank_host_threads(world)  # an earlier oracle leg may have taken every core for rank 0
     import torch.distributed as dist
     from lorb_slam_b200 import capi, sharding, synth
-    steps = steps or args.steps
+    steps = args.steps
     warmup = max(3, min(args.warmup, 3))
     ctx = capi.Context(local)
     # the communicator exists at world 1 as well: the sharded code path (separate control kernel,
@@ -804,6 +851,8 @@ def run_ba_large(args, rank, world, local, steps=None, want_cpu=True):
     clocks = sampler.stop() if rank == 0 else None
     dt_max = _max_over_ranks(dt, world, local)
     cams_res, pts_res = prob.download()
+    if rank == 0:
+        OUTPUTS.update(ba_large_cams=cams_res, ba_large_points=pts_res, ba_large_summary=_ba_summary_rows([s]))
     # ---- parity inside the run: the un-sharded solve of the whole problem on rank 0 (at world 1: the
     # sharded code path over a one-rank communicator) must give the same cameras / points
     # Both sides run under Ceres' default tolerances (at most 10 iterations): the timed runs force all 10
@@ -846,14 +895,13 @@ def run_ba_large(args, rank, world, local, steps=None, want_cpu=True):
     # ---- e2e: the host-buffer call every step (upload, device work lists, solve, download): lorb_ba_local
     # on one GPU, lorb_ba_local_shard (this rank's shard, collective) on several.
     _barrier(world)
-    n_e2e = max(1, steps // 2)
     e2e_call = ctx.ba_local if world == 1 else ctx.ba_local_shard
     e2e_call(sh, opt)  # first call sizes the grow-only buffers of the ctx
     _barrier(world)
     t0 = time.perf_counter()
-    for _ in range(n_e2e):
+    for _ in range(steps):
         e2e_call(sh, opt)
-    e2e = _max_over_ranks((time.perf_counter() - t0) / n_e2e, world, local)
+    e2e = _max_over_ranks((time.perf_counter() - t0) / steps, world, local)
     O = pb["O"]
     value = steps * O * s["iterations"] / dt_max
     res = None
@@ -904,7 +952,13 @@ def main():
     ap.add_argument("--large-points", type=int, default=200000)
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "lorb":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl lorb)")
     args.warmup = max(args.warmup, 3) if args.impl == "lorb" else args.warmup
 
     if args.impl == "reference":
@@ -937,14 +991,15 @@ def main():
                 res["full_sweep"] = f
         del bank
         if args.workload == "all":
-            # the other two BASELINE metrics, same contract, shorter runs
-            sub_steps = max(2, min(args.steps, 5))
-            b = run_ba_batched(args, rank, world, local, steps=sub_steps, want_cpu=want_cpu)
-            l = run_ba_large(args, rank, world, local, steps=sub_steps, want_cpu=want_cpu)
+            # the other two BASELINE metrics, same contract
+            b = run_ba_batched(args, rank, world, local, want_cpu=want_cpu)
+            l = run_ba_large(args, rank, world, local, want_cpu=want_cpu)
             if rank == 0:
                 res["ba_batched"] = b
                 res["ba_large"] = l
     if rank == 0:
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs)
         print(json.dumps(res), flush=True)
     if world > 1:
         import torch.distributed as dist

@@ -73,6 +73,33 @@ def test_oracle_image_ops_match_cv2(c):
     OC.check_stages_against_cv2(_oracle_stages, c)
 
 
+@pytest.mark.parametrize("c", RC.ORB_EXTRACT, ids=[c[0] for c in RC.ORB_EXTRACT])
+def test_oracle_extract_matches_reference_golden(c):
+    """The whole extractor assembled from the restated stages == the reference's own
+    ORBextractor::operator() outputs (ext/<case>/*): the stand-in the GPU tests compare fresh frames
+    with where oracle/_ref is not built."""
+    OC.check_extract(lambda img, nf: OC.oracle_extract(img, nfeatures=nf), c)
+
+
+@pytest.mark.parametrize("kw", [dict(nfeatures=1000, scale_factor=1.2, nlevels=8), dict(nfeatures=64, nlevels=8),
+                                dict(nfeatures=3000, nlevels=6), dict(nfeatures=1000, scale_factor=1.5, nlevels=4),
+                                dict(nfeatures=100, nlevels=1)], ids=["default", "n64", "n3000_l6", "sf1.5_l4", "l1"])
+def test_level_plan_restatement(kw):
+    """OC.level_plan (the constructor's tables, restated for the oracle extractor) == the library's
+    host arithmetic, over frame sizes including odd ones."""
+    for width, height in ((640, 480), (752, 480), (161, 241), (1280, 240), (1241, 376), (97, 113)):
+        prm = capi.OrbParams(kw["nfeatures"], kw.get("scale_factor", 1.2), kw["nlevels"], 20, 7)
+        nl = kw["nlevels"]
+        w, h, nf = (np.zeros(nl, np.int32) for _ in range(3))
+        sf = np.zeros(nl, np.float32)
+        p = lambda a: a.ctypes.data_as(C.c_void_p)  # noqa: E731
+        rc = capi.load_library().lorb_orb_level_sizes(C.byref(prm), width, height, p(w), p(h), p(nf), p(sf))
+        if rc != 0:
+            continue  # a level smaller than the blur kernel: refused by the library, never extracted
+        ow, oh, onf, osf = OC.level_plan(width, height, kw["nfeatures"], kw.get("scale_factor", 1.2), nl)
+        assert (ow, oh, onf) == (list(w), list(h), list(nf)) and np.array_equal(osf, sf), (width, height)
+
+
 def test_level_plan():
     w, h, nf, sf = capi_level_sizes(640, 480)
     assert list(w) == [640, 533, 444, 370, 309, 257, 214, 179] and list(h) == [480, 400, 333, 278, 231, 193, 161, 134]

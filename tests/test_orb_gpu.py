@@ -105,13 +105,11 @@ def test_cuda_stages_fresh(ctx, seed, w, h):
 
 @pytest.mark.parametrize("seed", range(3))
 def test_cuda_orb_extract_fresh_vs_reference(ctx, seed):
-    """Against the compiled reference itself when its library travelled with the snapshot."""
-    from oracle import reflib
-    if not reflib.available():
-        pytest.skip("oracle/_ref not built")
+    """Against the compiled reference where oracle/_ref is built, else against the oracle extractor
+    (pinned to the reference's outputs by test_orb_cpu)."""
     img = synth.make_orb_image(40 + seed, 640 + 16 * seed, 480)
     for nf in (1000, 150):
-        a, b = ctx.orb_extract(img, OC.pattern(), nfeatures=nf), reflib.orb_extract(img, nfeatures=nf)
+        a, b = ctx.orb_extract(img, OC.pattern(), nfeatures=nf), OC.reference_extract(img, nfeatures=nf)
         assert a["n"] == b["n"]
         for f in ("x", "y", "octave", "angle", "response", "size", "desc"):
             assert np.array_equal(a[f], b[f]), f
@@ -183,15 +181,12 @@ def test_stereo_frame_front_end(ctx, seed):
                          ids=["one_level", "sf1.5", "th40_12", "th9_9", "n64", "n3000_l6"])
 def test_cuda_orb_extract_parameters_vs_reference(ctx, kw):
     """Non-default ORBextractor constructor arguments, and a strided (non-contiguous) input image."""
-    from oracle import reflib
-    if not reflib.available():
-        pytest.skip("oracle/_ref not built")
     img = synth.make_orb_image(77, 700, 500)
     view = img[6:486, 20:660]  # 640x480 window of a 700-px-wide buffer: step 700
     assert not view.flags["C_CONTIGUOUS"]
     prm = dict(nfeatures=1000, scale_factor=1.2, nlevels=8, ini_th=20, min_th=7)
     prm.update(kw)
-    b = reflib.orb_extract(np.ascontiguousarray(view), **prm)
+    b = OC.reference_extract(np.ascontiguousarray(view), **prm)
     cap = prm["nfeatures"] + 64
     # the ctypes wrapper makes arrays contiguous; call the C ABI with the strided view directly
     import ctypes as C
@@ -266,10 +261,8 @@ def test_cuda_orb_extract_soak_vs_reference(ctx):
     """A slice of profiles/scripts/orb_soak.py (300 frames there: 0 differ): varied frame sizes,
     textures (low contrast, pure noise, half flat), budgets, level counts and thresholds, each
     bit-exact against the compiled reference -- including wide frames with small budgets, which
-    return more keypoints than nfeatures + a few (lorb_orb_max_keypoints)."""
-    from oracle import reflib
-    if not reflib.available():
-        pytest.skip("oracle/_ref not built")
+    return more keypoints than nfeatures + a few (lorb_orb_max_keypoints).  Where oracle/_ref is not
+    built, the oracle extractor stands in for the reference."""
     rng = np.random.default_rng(99)
     over = 0
     for f in range(28):
@@ -284,7 +277,7 @@ def test_cuda_orb_extract_soak_vs_reference(ctx):
             img[:, : w // 2] = 100
         nf, nl = int(rng.choice([100, 500, 2000])), int(rng.choice([4, 8]))
         a = ctx.orb_extract(img, OC.pattern(), nfeatures=nf, nlevels=nl)
-        b = reflib.orb_extract(img, nfeatures=nf, nlevels=nl)
+        b = OC.reference_extract(img, nfeatures=nf, nlevels=nl)
         assert a["n"] == b["n"] <= ctx.orb_max_keypoints(w, h, nfeatures=nf, nlevels=nl), (f, w, h, nf, nl)
         for k in ("x", "y", "octave", "angle", "response", "size", "desc"):
             assert np.array_equal(a[k], b[k]), (f, k)
@@ -292,5 +285,5 @@ def test_cuda_orb_extract_soak_vs_reference(ctx):
     # the case a fixed "nfeatures + 64" capacity misses: a wide frame with a small budget keeps 4 nodes
     # per initial quadtree column on every level
     img = synth.make_orb_image(640, 1280, 240)
-    a, b = ctx.orb_extract(img, OC.pattern(), nfeatures=100), reflib.orb_extract(img, nfeatures=100)
+    a, b = ctx.orb_extract(img, OC.pattern(), nfeatures=100), OC.reference_extract(img, nfeatures=100)
     assert a["n"] == b["n"] > 100 + 64 and np.array_equal(a["desc"], b["desc"]) and np.array_equal(a["x"], b["x"])
