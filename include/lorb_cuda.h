@@ -472,7 +472,7 @@ enum {
 };
 
 typedef struct lorb_ba_summary {
-  double initial_cost;  /* 1/2 sum r^2 at the input */
+  double initial_cost;  /* 1/2 sum rho(|r|^2) at the input (rho = identity unless a loss is set) */
   double final_cost;
   double final_radius;
   double final_gradient_max_norm;
@@ -485,6 +485,31 @@ typedef struct lorb_ba_summary {
 void lorb_ba_default_options(lorb_ba_options* opt);
 
 /*
+ * Robust loss of every BA solve on a ctx (beyond the reference, which passes no loss to
+ * AddResidualBlock; Ceres LossFunction semantics).  With s = |r|^2 of one observation's 2-vector
+ * residual, a = scale, b = a^2, c = 1/b:
+ *   LORB_LOSS_TRIVIAL   rho(s) = s                      (default: plain least squares, the reference)
+ *   LORB_LOSS_HUBER     rho(s) = s (s <= b), 2 a sqrt(s) - b (s > b)        (ceres::HuberLoss)
+ *   LORB_LOSS_SOFTLONE  rho(s) = 2 b (sqrt(1 + s c) - 1)                    (ceres::SoftLOneLoss)
+ *   LORB_LOSS_CAUCHY    rho(s) = b log(1 + s c)                             (ceres::CauchyLoss)
+ * The solvers minimise 1/2 sum rho(s); residuals and Jacobians are scaled by sqrt(rho'(s)) at the
+ * point of linearisation (Ceres' Corrector, whose curvature term vanishes for these losses), so the
+ * gradient, the normal equations, the Jacobi scaling and the model decrease are those of the
+ * corrected problem.  Summary costs and gradient norms are those of the robust problem.
+ * lorb_ba_set_loss(ctx, NULL) restores the trivial loss.  It returns < 0 and leaves the ctx as it
+ * was for an unknown kind, or for a scale that is not finite and > 0 when the kind is not trivial
+ * (the trivial loss ignores the scale).  The setting holds until the next call on that ctx.
+ */
+enum { LORB_LOSS_TRIVIAL = 0, LORB_LOSS_HUBER = 1, LORB_LOSS_SOFTLONE = 2, LORB_LOSS_CAUCHY = 3 };
+typedef struct lorb_ba_loss {
+  int kind;     /* LORB_LOSS_* */
+  int reserved;
+  double scale; /* a > 0, in pixels */
+} lorb_ba_loss;
+int lorb_ba_set_loss(lorb_ctx* ctx, const lorb_ba_loss* loss);
+int lorb_ba_get_loss(lorb_ctx* ctx, lorb_ba_loss* loss);
+
+/*
  * BA::ProjectPoseOptimization (reference src/bundle_adjust.cpp:158-202):
  * 6-dof pose (angle-axis R, translation T) of one frame against fixed 3-D
  * points, PoseCost residuals (src/bundle_adjust.cpp:22-64 — including its use
@@ -493,6 +518,7 @@ void lorb_ba_default_options(lorb_ba_options* opt);
  *   uv [n x 2] float   Frame::GetKp2d(i)
  *   K = {fx, fy, cx, cy} float (fy is unused by PoseCost; kept for symmetry)
  *   rt [6] double in/out: (R0,R1,R2,T0,T1,T2)
+ * Minimises with the ctx's robust loss (lorb_ba_set_loss).
  */
 int lorb_ba_pose_only(lorb_ctx* ctx, int n, const float* xw, const float* uv, const float* K,
                       double* rt, const lorb_ba_options* opt, lorb_ba_summary* summary);
@@ -507,6 +533,8 @@ int lorb_ba_pose_only(lorb_ctx* ctx, int n, const float* xw, const float* uv, co
  *                (:68-113, :288-289)
  *   K = {fx, fy, cx, cy} of pCurrFrame->mpCamera
  * No parameter block is held constant (the reference holds none).
+ * Minimises with the ctx's robust loss (lorb_ba_set_loss), in-window and fixed
+ * observations alike.
  */
 int lorb_ba_local(lorb_ctx* ctx, int C, double* cams, int P, double* pts, int O, const int* obs_cam,
                   const int* obs_pt, const float* obs_uv, int F, const int* fix_pt,
@@ -518,6 +546,7 @@ int lorb_ba_local(lorb_ctx* ctx, int C, double* cams, int P, double* pts, int O,
  * arrays hold THIS RANK'S points with all their observations (lorb_shard_range / the natural layout
  * of a distributed map) and every camera; a collective call over the communicator of lorb_dist_init.
  * On return cams holds all C cameras (identical on every rank), pts this rank's points.
+ * Every rank must have set the same robust loss (lorb_ba_set_loss) on its ctx.
  */
 int lorb_ba_local_shard(lorb_ctx* ctx, int C, double* cams, int P, double* pts, int O, const int* obs_cam,
                         const int* obs_pt, const float* obs_uv, int F, const int* fix_pt,
@@ -530,7 +559,8 @@ int lorb_ba_local_shard(lorb_ctx* ctx, int C, double* cams, int P, double* pts, 
  *   obs[obs_off[w] .. obs_off[w+1])  with obs_cam / obs_pt LOCAL to the window,
  *   fixed observations [fix_off[w] .. fix_off[w+1]) likewise (fix_off may be
  *   NULL when there are none).
- * Every window runs its own LM loop (own trust region, own termination).
+ * Every window runs its own LM loop (own trust region, own termination), all
+ * with the ctx's robust loss (lorb_ba_set_loss).
  */
 int lorb_ba_local_batched(lorb_ctx* ctx, int n_windows, const int* cam_off, double* cams,
                           const int* pt_off, double* pts, const int* obs_off, const int* obs_cam,
@@ -593,7 +623,9 @@ int lorb_ba_problem_reset(lorb_ba_problem* p);
 /* Run LM on the resident problem.  If the ctx has a distributed group
  * (lorb_dist_init) and `sharded` != 0, the points/observations given to this
  * rank are its shard, cameras are replicated, and the reduced camera system is
- * all-reduced over NCCL every iteration (SURVEY §8(e)). */
+ * all-reduced over NCCL every iteration (SURVEY §8(e)).  The robust loss is the
+ * one set on the problem's ctx when this is called, not at creation, so one
+ * resident problem can be re-solved under different losses. */
 int lorb_ba_problem_solve(lorb_ba_problem* p, const lorb_ba_options* opt, int sharded,
                           lorb_ba_summary* summary);
 int lorb_ba_problem_download(lorb_ba_problem* p, double* cams, double* pts);

@@ -16,6 +16,9 @@ LIB_PATH = os.path.join(_HERE, "lib", "liblorb_cuda.so")
 OK = 0
 CROSSCHECK_MUTUAL, CROSSCHECK_LEGACY = 0, 1
 SWEEP_POPC, SWEEP_TENSOR, SWEEP_DEFAULT = 0, 1, -1
+# robust losses of the BA solvers (lorb_ba_set_loss): plain least squares, ceres::HuberLoss,
+# SoftLOneLoss, CauchyLoss
+LOSS_TRIVIAL, LOSS_HUBER, LOSS_SOFTLONE, LOSS_CAUCHY = 0, 1, 2, 3
 TERMINATION = {0: "NO_CONVERGENCE", 1: "CONV_FUNCTION", 2: "CONV_GRADIENT", 3: "CONV_PARAMETER",
                4: "CONV_RADIUS", 5: "FAILURE"}
 
@@ -31,7 +34,8 @@ EXPORTS = [
     "lorb_orb_extract", "lorb_orb_level_sizes", "lorb_orb_stages", "lorb_stereo_frame", "lorb_orb_distribute", "lorb_orb_max_keypoints",
     "lorb_ba_default_options", "lorb_ba_pose_only", "lorb_ba_local", "lorb_ba_local_batched", "lorb_ba_local_shard",
     "lorb_ba_problem_create", "lorb_ba_problem_create_batched", "lorb_ba_problem_create_sharded", "lorb_shard_range", "lorb_ba_shard_points", "lorb_set_host_threads", "lorb_ba_problem_reset", "lorb_ba_problem_solve",
-    "lorb_ba_problem_download", "lorb_ba_problem_destroy", "lorb_dist_get_unique_id",
+    "lorb_ba_problem_download", "lorb_ba_problem_destroy", "lorb_ba_set_loss", "lorb_ba_get_loss",
+    "lorb_dist_get_unique_id",
     "lorb_dist_init", "lorb_dist_finalize", "lorb_dist_allreduce_f64", "lorb_microbench_popc",
     "lorb_microbench_fp64", "lorb_microbench_tensor_i8", "lorb_ctx_profile", "lorb_ctx_profile_read",
 ]
@@ -49,6 +53,10 @@ class BAOptions(C.Structure):
                 ("max_trust_region_radius", C.c_double), ("min_trust_region_radius", C.c_double),
                 ("min_relative_decrease", C.c_double), ("min_lm_diagonal", C.c_double),
                 ("max_lm_diagonal", C.c_double)]
+
+
+class BALoss(C.Structure):
+    _fields_ = [("kind", C.c_int), ("reserved", C.c_int), ("scale", C.c_double)]
 
 
 class BASummary(C.Structure):
@@ -265,6 +273,16 @@ class Context:
         """SWEEP_POPC / SWEEP_TENSOR / SWEEP_DEFAULT (or "popc" / "tensor" / "default")."""
         impl = {"popc": SWEEP_POPC, "tensor": SWEEP_TENSOR, "default": SWEEP_DEFAULT}.get(impl, impl)
         _check(self._lib.lorb_sweep_set_impl(self._h, int(impl)))
+
+    def ba_set_loss(self, kind, scale=1.0):
+        """Robust loss (LOSS_*, scale a in pixels) of every later BA solve on this ctx."""
+        _check(self._lib.lorb_ba_set_loss(self._h, C.byref(BALoss(int(kind), 0, float(scale)))))
+
+    def ba_get_loss(self):
+        """-> (kind, scale) of the ctx's BA loss."""
+        lo = BALoss()
+        _check(self._lib.lorb_ba_get_loss(self._h, C.byref(lo)))
+        return lo.kind, lo.scale
 
     def bank_upload(self, bank):
         bank = _arr(bank, np.uint8)

@@ -71,6 +71,8 @@ struct BADev {
   const int4* pairs;      // (point, observation i, observation j, 0) grouped by camera block
   const int4* pair_items; // (ci, cj, start in pairs, length)
   int n_cam_items, n_pair_items;
+  int loss_kind;         // LORB_LOSS_* of the solve (read by the ROBUST kernel instantiations only)
+  double loss_scale;
 };
 
 __device__ __forceinline__ int upper_idx(int a, int b) {  // a <= b, 6x6
@@ -109,10 +111,14 @@ __global__ void ba_camrot_kernel(const BADev* __restrict__ probs, int which /*0 
 }
 
 // Observation of point X by window camera `cam` (>= 0) at pixel uv, with scaled Jacobians.
+// ROBUST: r and the Jacobians come out corrected by the solve's loss (robust_correct) and *rho, when
+// given, receives rho(|r|^2); the kernels are instantiated with ROBUST = false for plain least
+// squares, which keeps that path exactly the code it was.
+template <bool ROBUST = false>
 __device__ __forceinline__ void eval_obs_cam(const BADev& p, const double* __restrict__ cams,
                                              const double* __restrict__ camrot, int cam, float2 uv,
                                              const double X[3], const double sp[3], double r[2], double Jc[12],
-                                             double Jp[6]) {
+                                             double Jp[6], double* rho = nullptr) {
   const double* t = cams + 6 * cam + 3;
   const double tt[3] = {t[0], t[1], t[2]};
   obs_eval<true, true>(camrot + CAMROT * cam, tt, X, p.K, (double)uv.x, (double)uv.y, r, Jc, Jp);
@@ -127,17 +133,22 @@ __device__ __forceinline__ void eval_obs_cam(const BADev& p, const double* __res
     Jp[a] *= sp[a];
     Jp[3 + a] *= sp[a];
   }
+  if (ROBUST) {
+    const double q = robust_correct(p.loss_kind, p.loss_scale, r, Jc, Jp);
+    if (rho) *rho = q;
+  }
 }
 
-// Evaluate observation `o` of point X with scaled Jacobians.
+// Evaluate observation `o` of point X with scaled Jacobians (ROBUST, rho: as eval_obs_cam).
+template <bool ROBUST = false>
 __device__ __forceinline__ int eval_obs(const BADev& p, const double* __restrict__ cams,
                                         const double* __restrict__ camrot, int o, const double X[3],
                                         const double sp[3], double r[2], double Jc[12],
-                                        double Jp[6]) {
+                                        double Jp[6], double* rho = nullptr) {
   const int cam = p.obs_cam[o];
   const float2 uv = p.obs_uv[o];
   if (cam >= 0) {
-    eval_obs_cam(p, cams, camrot, cam, uv, X, sp, r, Jc, Jp);
+    eval_obs_cam<ROBUST>(p, cams, camrot, cam, uv, X, sp, r, Jc, Jp, rho);
     return cam;
   }
   const double* f = p.fixrt + 12 * (size_t)(-1 - cam);
@@ -147,6 +158,10 @@ __device__ __forceinline__ int eval_obs(const BADev& p, const double* __restrict
   for (int a = 0; a < 3; a++) {
     Jp[a] *= sp[a];
     Jp[3 + a] *= sp[a];
+  }
+  if (ROBUST) {
+    const double q = robust_correct(p.loss_kind, p.loss_scale, r, nullptr, Jp);
+    if (rho) *rho = q;
   }
   return cam;
 }
@@ -172,9 +187,10 @@ __device__ __forceinline__ void cs_fill(const BADev& p, const double* __restrict
 }
 
 // eval_obs with the window's cameras in shared memory (same arithmetic, same order).
+template <bool ROBUST = false>
 __device__ __forceinline__ int eval_obs_cs(const BADev& p, const double* __restrict__ cs, int stride, int o,
                                            const double X[3], const double sp[3], double r[2], double Jc[12],
-                                           double Jp[6]) {
+                                           double Jp[6], double* rho = nullptr) {
   const int cam = p.obs_cam[o];
   const float2 uv = p.obs_uv[o];
   if (cam >= 0) {
@@ -196,7 +212,20 @@ __device__ __forceinline__ int eval_obs_cs(const BADev& p, const double* __restr
     Jp[a] *= sp[a];
     Jp[3 + a] *= sp[a];
   }
+  if (ROBUST) {
+    const double q = robust_correct(p.loss_kind, p.loss_scale, r, cam >= 0 ? Jc : nullptr, Jp);
+    if (rho) *rho = q;
+  }
   return cam;
+}
+
+// Candidate cost of one observation with squared residual norm s: rho(s) under the solve's loss.
+template <bool ROBUST>
+__device__ __forceinline__ double obs_rho(const BADev& p, double s) {
+  if (!ROBUST) return s;
+  double rho, rho1;
+  loss_eval(p.loss_kind, p.loss_scale, s, rho, rho1);
+  return rho;
 }
 
 // |g_a / s_a| of the unscaled point gradient, coordinate a = lane of the point's group: the three
@@ -275,7 +304,7 @@ __device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double
                : "d"(a), "d"(b));
 }
 
-template <bool FULL, int ACC>
+template <bool FULL, int ACC, bool ROBUST = false>
 __global__ void __launch_bounds__(BA_THREADS)
     ba_build_kernel(const BADev* __restrict__ probs, lorb_ba_options opt, int force) {
   const BADev p = probs[blockIdx.y];
@@ -330,8 +359,9 @@ __global__ void __launch_bounds__(BA_THREADS)
       const int o = s + rd * 8 + gl;
       has = o < e;
       if (has) {
-        cam = eval_obs(p, cams, camrot, o, X, sp, r, Jc, Jp);
-        cost_acc += r[0] * r[0] + r[1] * r[1];
+        double rho;
+        cam = eval_obs<ROBUST>(p, cams, camrot, o, X, sp, r, Jc, Jp, &rho);
+        cost_acc += ROBUST ? rho : r[0] * r[0] + r[1] * r[1];
         h[0] += Jp[0] * Jp[0] + Jp[3] * Jp[3];
         h[1] += Jp[0] * Jp[1] + Jp[3] * Jp[4];
         h[2] += Jp[0] * Jp[2] + Jp[3] * Jp[5];
@@ -395,7 +425,7 @@ __global__ void __launch_bounds__(BA_THREADS)
       int ci = -1;
       double Wi[18], Yi[18];
       if (rounds > 1 || ri > 0) {
-        if (has_i) ci = eval_obs(p, cams, camrot, oi, X, sp, r, Jc, Jp);
+        if (has_i) ci = eval_obs<ROBUST>(p, cams, camrot, oi, X, sp, r, Jc, Jp);
       } else {
         ci = has ? cam : -1;  // single round: Jacobians of phase 1 are still live
       }
@@ -427,7 +457,7 @@ __global__ void __launch_bounds__(BA_THREADS)
           int cj = -1;
           if (oj < e) {
             double r2[2], Jc2[12], Jp2[6];
-            cj = eval_obs(p, cams, camrot, oj, X, sp, r2, Jc2, Jp2);
+            cj = eval_obs<ROBUST>(p, cams, camrot, oj, X, sp, r2, Jc2, Jp2);
             if (cj >= 0) {
 #pragma unroll
               for (int a = 0; a < 6; a++)
@@ -593,7 +623,7 @@ __device__ __forceinline__ void dense_reduce(double* __restrict__ Sbuf, double* 
   }
 }
 
-template <bool FULL>
+template <bool FULL, bool ROBUST = false>
 __global__ void __launch_bounds__(DP_THREADS)
     ba_build_dense_kernel(const BADev* __restrict__ probs, lorb_ba_options opt, int force) {
   const BADev p = probs[blockIdx.y];
@@ -650,8 +680,9 @@ __global__ void __launch_bounds__(DP_THREADS)
       const int o = s + rd * 8 + gl;
       has = o < e;
       if (has) {
-        cam = eval_obs_cs(p, cs, CS_BUILD, o, X, sp, r, Jc, Jp);
-        cost_acc += r[0] * r[0] + r[1] * r[1];
+        double rho;
+        cam = eval_obs_cs<ROBUST>(p, cs, CS_BUILD, o, X, sp, r, Jc, Jp, &rho);
+        cost_acc += ROBUST ? rho : r[0] * r[0] + r[1] * r[1];
         h[0] += Jp[0] * Jp[0] + Jp[3] * Jp[3];
         h[1] += Jp[0] * Jp[1] + Jp[3] * Jp[4];
         h[2] += Jp[0] * Jp[2] + Jp[3] * Jp[5];
@@ -720,7 +751,7 @@ __global__ void __launch_bounds__(DP_THREADS)
         const bool has_i = oi < e;
         int ci = -1;
         if (rounds > 1) {
-          if (has_i) ci = eval_obs_cs(p, cs, CS_BUILD, oi, X, sp, r, Jc, Jp);
+          if (has_i) ci = eval_obs_cs<ROBUST>(p, cs, CS_BUILD, oi, X, sp, r, Jc, Jp);
         } else {
           ci = has ? cam : -1;  // single round: the Jacobians of phase 1 are still live
         }
@@ -840,6 +871,7 @@ __global__ void __launch_bounds__(DP_THREADS)
 // list): one warp accumulates H_cc (21), g_c (6) and the Schur right-hand side
 // W H_pp^-1 g_p (6) of its slice in registers, reduces by shuffles and issues 33
 // atomics per item.
+template <bool ROBUST = false>
 __global__ void __launch_bounds__(256)
     ba_cam_rows_kernel(const BADev* __restrict__ probs, int full, int force) {
   const BADev p = probs[blockIdx.y];
@@ -868,7 +900,7 @@ __global__ void __launch_bounds__(256)
       X[a] = pts[3 * (size_t)pt + a];
       sp[a] = p.scale_p[3 * (size_t)pt + a];
     }
-    eval_obs_cam(p, cams, camrot, it.x, uv, X, sp, r, Jc, Jp);
+    eval_obs_cam<ROBUST>(p, cams, camrot, it.x, uv, X, sp, r, Jc, Jp);
     int k = 0;
 #pragma unroll
     for (int a = 0; a < 6; a++) {
@@ -913,6 +945,7 @@ __global__ void __launch_bounds__(256)
 // of one point with camera(i) = ci, camera(j) = cj.  One warp accumulates
 // sum Y_i W_j^T (6x6) in registers over its slice, reduces by shuffles and
 // subtracts it from S with 36 atomics per item (an item is <= 2048 records).
+template <bool ROBUST = false>
 __global__ void __launch_bounds__(256)
     ba_schur_pairs_kernel(const BADev* __restrict__ probs) {
   const BADev p = probs[blockIdx.y];
@@ -944,7 +977,7 @@ __global__ void __launch_bounds__(256)
     }
     const double* hi = p.pt_hinv + 6 * (size_t)pt;
     const double h0 = hi[0], h1 = hi[1], h2 = hi[2], h3 = hi[3], h4 = hi[4], h5 = hi[5];
-    eval_obs_cam(p, cams, camrot, it.x, uvi, X, sp, r, Jc, Jp);
+    eval_obs_cam<ROBUST>(p, cams, camrot, it.x, uvi, X, sp, r, Jc, Jp);
 #pragma unroll
     for (int a = 0; a < 6; a++) {
       const double w0 = Jc[a] * Jp[0] + Jc[6 + a] * Jp[3];
@@ -954,7 +987,7 @@ __global__ void __launch_bounds__(256)
       Y[3 * a + 1] = w0 * h1 + w1 * h3 + w2 * h4;
       Y[3 * a + 2] = w0 * h2 + w1 * h4 + w2 * h5;
     }
-    if (oj != oi) eval_obs_cam(p, cams, camrot, it.y, uvj, X, sp, r, Jc, Jp);
+    if (oj != oi) eval_obs_cam<ROBUST>(p, cams, camrot, it.y, uvj, X, sp, r, Jc, Jp);
 #pragma unroll
     for (int b = 0; b < 6; b++) {
       const double w0 = Jc[b] * Jp[0] + Jc[6 + b] * Jp[3];
@@ -2245,7 +2278,8 @@ __device__ __forceinline__ void lm_control(const BADev& p, const lorb_ba_options
   *p.st = loc;
 }
 
-template <bool CS>  // CS: every window of the launch has <= CS_MAX_CAMS cameras, kept in shared memory
+// CS: every window of the launch has <= CS_MAX_CAMS cameras, kept in shared memory
+template <bool CS, bool ROBUST = false>
 __global__ void __launch_bounds__(BA_THREADS, 2)  // latency-bound gathers: two CTAs per SM (ncu: long_scoreboard)
     ba_backsub_kernel(const BADev* __restrict__ probs, lorb_ba_options opt, int fuse_control,
                       int* __restrict__ n_active) {
@@ -2311,7 +2345,8 @@ __global__ void __launch_bounds__(BA_THREADS, 2)  // latency-bound gathers: two 
       const int o = s + rd * 8 + gl;
       has = o < e;
       if (has) {
-        cam = CS ? eval_obs_cs(p, cs, CS_BACKSUB, o, X, sp, r, Jc, Jp) : eval_obs(p, cams, camrot, o, X, sp, r, Jc, Jp);
+        cam = CS ? eval_obs_cs<ROBUST>(p, cs, CS_BACKSUB, o, X, sp, r, Jc, Jp)
+                 : eval_obs<ROBUST>(p, cams, camrot, o, X, sp, r, Jc, Jp);
         jcy[0] = jcy[1] = 0;
         if (cam >= 0) {
           const double* ycam = CS ? cs + cam * CS_BACKSUB + CS_BUILD : yc + 6 * cam;
@@ -2352,7 +2387,8 @@ __global__ void __launch_bounds__(BA_THREADS, 2)  // latency-bound gathers: two 
       const int o = s + rd * 8 + gl;
       if (o < e) {
         if (rounds > 1) {
-          cam = CS ? eval_obs_cs(p, cs, CS_BACKSUB, o, X, sp, r, Jc, Jp) : eval_obs(p, cams, camrot, o, X, sp, r, Jc, Jp);
+          cam = CS ? eval_obs_cs<ROBUST>(p, cs, CS_BACKSUB, o, X, sp, r, Jc, Jp)
+                 : eval_obs<ROBUST>(p, cams, camrot, o, X, sp, r, Jc, Jp);
           jcy[0] = jcy[1] = 0;
           if (cam >= 0) {
             const double* ycam = CS ? cs + cam * CS_BACKSUB + CS_BUILD : yc + 6 * cam;
@@ -2371,11 +2407,11 @@ __global__ void __launch_bounds__(BA_THREADS, 2)  // latency-bound gathers: two 
           const double* rc = CS ? cs + cam * CS_BACKSUB + 51 : camrot_c + CAMROT * cam;
           const double* t = CS ? cs + cam * CS_BACKSUB + 60 : cams_c + 6 * cam + 3;
           const double tt[3] = {t[0], t[1], t[2]};
-          cost_acc += obs_cost(rc, tt, Xc, p.K, (double)uv.x, (double)uv.y);
+          cost_acc += obs_rho<ROBUST>(p, obs_cost(rc, tt, Xc, p.K, (double)uv.x, (double)uv.y));
         } else {
           const double* f = p.fixrt + 12 * (size_t)(-1 - cam);
           const double tt[3] = {f[9], f[10], f[11]};
-          cost_acc += obs_cost(f, tt, Xc, p.K, (double)uv.x, (double)uv.y);
+          cost_acc += obs_rho<ROBUST>(p, obs_cost(f, tt, Xc, p.K, (double)uv.x, (double)uv.y));
         }
       }
     }
@@ -3178,6 +3214,22 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
       LORB_CUDA_TRY(cudaMemcpyAsync(pb->descs.p, &h0, sizeof(BADev), cudaMemcpyHostToDevice, c->stream));
     }
   }
+  // the robust loss is the ctx's at solve time: every window's descriptor carries it
+  const lorb_ba_loss loss = c->ba_loss;
+  const bool robust = loss.kind != LORB_LOSS_TRIVIAL;
+  {
+    bool changed = false;
+    for (BADev& d : pb->h_dev) {
+      changed |= d.loss_kind != loss.kind || d.loss_scale != loss.scale;
+      d.loss_kind = loss.kind;
+      d.loss_scale = loss.scale;
+    }
+    if (changed)
+      LORB_CUDA_TRY(cudaMemcpyAsync(pb->descs.p, pb->h_dev.data(), sizeof(BADev) * (size_t)nw,
+                                    cudaMemcpyHostToDevice, c->stream));
+  }
+  // kernel instantiation for the loss: ROBUST = false is plain least squares, unchanged
+#define LORB_BA_K(K_, ...) (robust ? K_<__VA_ARGS__, true> : K_<__VA_ARGS__, false>)
   const int gx_pts = std::max(1, std::min((pb->maxP + 31) / 32, std::max(1, c->sm_count * 8 / nw)));
   const dim3 grid_pts(gx_pts, nw);
   // back-substitution with the cameras in shared memory: two CTAs per SM must fit (C <= 203); a CTA
@@ -3185,7 +3237,7 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
   const size_t backsub_smem = (size_t)pb->maxC * CS_BACKSUB * 8;
   const bool backsub_cs = backsub_smem <= 100 * 1024;
   if (backsub_cs && backsub_smem > 40 * 1024)
-    LORB_CUDA_TRY(cudaFuncSetAttribute(ba_backsub_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    LORB_CUDA_TRY(cudaFuncSetAttribute(LORB_BA_K(ba_backsub_kernel, true), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)backsub_smem));
   const dim3 grid_backsub(backsub_smem > 16 * 1024 ? std::min(gx_pts, std::max(1, 2 * c->sm_count / nw)) : gx_pts, nw);
   const int ppc = DP_THREADS / 8;  // points per CTA round of the dense path
@@ -3224,15 +3276,15 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
                     : (acc_mode == 1 ? ((size_t)nmax * nmax + lin_small) * 8 + wsm_bytes : 0);
   const size_t smem_solve = ((size_t)nmax * nmax + 2 * (size_t)nmax + NB + (size_t)((nmax + NB - 1) / NB) * NB * (NB + 1)) * 8;
 #define LORB_BUILD_ATTR(FULL_, ACC_, BYTES_)                                                  \
-  LORB_CUDA_TRY(cudaFuncSetAttribute(ba_build_kernel<FULL_, ACC_>,                             \
+  LORB_CUDA_TRY(cudaFuncSetAttribute(LORB_BA_K(ba_build_kernel, FULL_, ACC_),                 \
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(BYTES_))); \
-  LORB_CUDA_TRY(cudaFuncSetAttribute(ba_build_kernel<FULL_, ACC_>,                             \
+  LORB_CUDA_TRY(cudaFuncSetAttribute(LORB_BA_K(ba_build_kernel, FULL_, ACC_),                 \
                                      cudaFuncAttributePreferredSharedMemoryCarveout,           \
                                      (int)cudaSharedmemCarveoutMaxShared))
   if (acc_mode == 2) {
-    LORB_CUDA_TRY(cudaFuncSetAttribute(ba_build_dense_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    LORB_CUDA_TRY(cudaFuncSetAttribute(LORB_BA_K(ba_build_dense_kernel, true), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)(DP_SMEM_DOUBLES * 8)));
-    LORB_CUDA_TRY(cudaFuncSetAttribute(ba_build_dense_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    LORB_CUDA_TRY(cudaFuncSetAttribute(LORB_BA_K(ba_build_dense_kernel, false), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)(DP_SMEM_DOUBLES * 8)));
   } else if (acc_mode == 1) {
     LORB_BUILD_ATTR(true, 1, smem_build_full);
@@ -3245,16 +3297,16 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
   auto launch_build = [&](bool full, int force) -> int {
     const size_t sm = full ? smem_build_full : smem_build_init;
 #define LORB_BUILD(FULL_, ACC_) \
-  LORB_LAUNCH(c, (ba_build_kernel<FULL_, ACC_>), grid_pts, BA_THREADS, sm, dp, opt, force)
+  LORB_LAUNCH(c, LORB_BA_K(ba_build_kernel, FULL_, ACC_), grid_pts, BA_THREADS, sm, dp, opt, force)
     if (acc_mode == 2) {
-      if (full) LORB_LAUNCH(c, ba_build_dense_kernel<true>, grid_dense, DP_THREADS, DP_SMEM_DOUBLES * 8, dp, opt, force);
-      else      LORB_LAUNCH(c, ba_build_dense_kernel<false>, grid_dense, DP_THREADS, DP_SMEM_DOUBLES * 8, dp, opt, force);
+      if (full) LORB_LAUNCH(c, LORB_BA_K(ba_build_dense_kernel, true), grid_dense, DP_THREADS, DP_SMEM_DOUBLES * 8, dp, opt, force);
+      else      LORB_LAUNCH(c, LORB_BA_K(ba_build_dense_kernel, false), grid_dense, DP_THREADS, DP_SMEM_DOUBLES * 8, dp, opt, force);
     } else if (acc_mode == 1) {
       if (full) LORB_BUILD(true, 1); else LORB_BUILD(false, 1);
     } else {
       // large path: point side, then camera side and Schur products from the work lists
-      if (full) LORB_LAUNCH(c, (ba_build_kernel<true, 3>), grid_pts, BA_THREADS, 0, dp, opt, force);
-      else      LORB_LAUNCH(c, (ba_build_kernel<false, 3>), grid_pts, BA_THREADS, 0, dp, opt, force);
+      if (full) LORB_LAUNCH(c, LORB_BA_K(ba_build_kernel, true, 3), grid_pts, BA_THREADS, 0, dp, opt, force);
+      else      LORB_LAUNCH(c, LORB_BA_K(ba_build_kernel, false, 3), grid_pts, BA_THREADS, 0, dp, opt, force);
       // camera rows (H_cc, g_c, Schur rhs) and Schur pairs (S) both need only the point side and write
       // disjoint outputs; both are latency-bound gathers, so the camera rows run on a side stream
       // beside the (six times longer) pair pass
@@ -3266,16 +3318,19 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
         }
         LORB_CUDA_TRY(cudaEventRecord(c->ba_ev[0], c->stream));
         LORB_CUDA_TRY(cudaStreamWaitEvent(c->ba_stream2, c->ba_ev[0], 0));
-        ba_cam_rows_kernel<<<dim3((pb->max_cam_items + 7) / 8, nw), 256, 0, c->ba_stream2>>>(dp, 1, force);
+        (robust ? ba_cam_rows_kernel<true> : ba_cam_rows_kernel<false>)
+            <<<dim3((pb->max_cam_items + 7) / 8, nw), 256, 0, c->ba_stream2>>>(dp, 1, force);
         c->launches++;
         LORB_CUDA_TRY(cudaGetLastError());
         LORB_CUDA_TRY(cudaEventRecord(c->ba_ev[1], c->ba_stream2));
       } else if (pb->max_cam_items > 0) {
-        LORB_LAUNCH(c, ba_cam_rows_kernel, dim3((pb->max_cam_items + 7) / 8, nw), 256, 0, dp,
+        LORB_LAUNCH(c, (robust ? ba_cam_rows_kernel<true> : ba_cam_rows_kernel<false>),
+                    dim3((pb->max_cam_items + 7) / 8, nw), 256, 0, dp,
                     full ? 1 : 0, force);
       }
       if (full && pb->max_pair_items > 0)
-        LORB_LAUNCH(c, ba_schur_pairs_kernel, dim3((pb->max_pair_items + 7) / 8, nw), 256, 0, dp);
+        LORB_LAUNCH(c, (robust ? ba_schur_pairs_kernel<true> : ba_schur_pairs_kernel<false>),
+                    dim3((pb->max_pair_items + 7) / 8, nw), 256, 0, dp);
       if (side) LORB_CUDA_TRY(cudaStreamWaitEvent(c->stream, c->ba_ev[1], 0));
     }
 #undef LORB_BUILD
@@ -3320,9 +3375,10 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
     prof_end(c, 2);
     prof_begin(c, 1);
     if (backsub_cs)
-      LORB_LAUNCH(c, ba_backsub_kernel<true>, grid_backsub, BA_THREADS, backsub_smem, dp, opt, fuse_control, d_active);
+      LORB_LAUNCH(c, LORB_BA_K(ba_backsub_kernel, true), grid_backsub, BA_THREADS, backsub_smem, dp, opt, fuse_control,
+                  d_active);
     else
-      LORB_LAUNCH(c, ba_backsub_kernel<false>, grid_pts, BA_THREADS, 0, dp, opt, fuse_control, d_active);
+      LORB_LAUNCH(c, LORB_BA_K(ba_backsub_kernel, false), grid_pts, BA_THREADS, 0, dp, opt, fuse_control, d_active);
     prof_end(c, 1);
     if (sharded) {
       prof_begin(c, 4);
@@ -3378,6 +3434,7 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
   }
   LORB_CUDA_TRY(cudaStreamSynchronize(s));
   return LORB_OK;
+#undef LORB_BA_K
 }
 
 // The host-buffer entry points (lorb_ba_local, lorb_ba_local_batched) reuse one

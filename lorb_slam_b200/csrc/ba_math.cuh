@@ -128,6 +128,55 @@ __device__ __forceinline__ void obs_eval(const double* __restrict__ rot, const d
   }
 }
 
+// Robust loss of one residual block, s = |r|^2, scale a (LORB_LOSS_*; Ceres HuberLoss,
+// SoftLOneLoss, CauchyLoss): rho(s) and rho'(s).  rho of soft-L1 and Cauchy is written without the
+// cancellation of 2b (sqrt(1 + s/b) - 1) and log(1 + s/b) for s << b (a scale far above the residuals
+// would otherwise leave five significant digits of the cost).  rho'' is not needed: it is <= 0 for all three, so
+// Ceres' Corrector drops its curvature term and scales r and J by sqrt(rho') alone.
+__device__ __forceinline__ void loss_eval(int kind, double a, double s, double& rho, double& rho1) {
+  const double b = a * a;
+  if (kind == LORB_LOSS_HUBER) {
+    if (s > b) {
+      const double r = sqrt(s);
+      rho = 2.0 * a * r - b;
+      rho1 = fmax(DBL_MIN, a / r);
+    } else {
+      rho = s;
+      rho1 = 1.0;
+    }
+  } else if (kind == LORB_LOSS_SOFTLONE) {
+    const double t = sqrt(1.0 + s * (1.0 / b));
+    rho = 2.0 * s / (t + 1.0);  // = 2b (t - 1)
+    rho1 = fmax(DBL_MIN, 1.0 / t);
+  } else if (kind == LORB_LOSS_CAUCHY) {
+    const double sum = 1.0 + s * (1.0 / b);
+    rho = b * log1p(s * (1.0 / b));
+    rho1 = fmax(DBL_MIN, 1.0 / sum);
+  } else {
+    rho = s;
+    rho1 = 1.0;
+  }
+}
+
+// Corrector of one observation: r and its Jacobian blocks (Jc: 12, Jp: 6; each may be null) are
+// scaled by sqrt(rho'(|r|^2)); returns rho(|r|^2), the observation's share of 2 * cost.
+__device__ __forceinline__ double robust_correct(int kind, double a, double r[2], double* Jc, double* Jp) {
+  double rho, rho1;
+  loss_eval(kind, a, r[0] * r[0] + r[1] * r[1], rho, rho1);
+  const double w = sqrt(rho1);
+  r[0] *= w;
+  r[1] *= w;
+  if (Jc) {
+#pragma unroll
+    for (int k = 0; k < 12; k++) Jc[k] *= w;
+  }
+  if (Jp) {
+#pragma unroll
+    for (int k = 0; k < 6; k++) Jp[k] *= w;
+  }
+  return rho;
+}
+
 // residual only (candidate cost)
 __device__ __forceinline__ double obs_cost(const double* __restrict__ R, const double t[3],
                                            const double X[3], const Intr& K, double u, double v) {

@@ -24,10 +24,12 @@ struct PoseShared {
   double red[POSE_THREADS / 32][NRED];
 };
 
-// sum r^2 (and optionally H, g) over all observations at pose `b`
-template <bool LIN>
+// sum r^2 (and optionally H, g) over all observations at pose `b`.  ROBUST: sum rho(|r|^2) and the
+// H, g of the residuals and Jacobians corrected by the loss (kind, a) (robust_correct).
+template <bool LIN, bool ROBUST>
 __device__ __forceinline__ void pose_pass(PoseShared& sm, int b, int n, const float* __restrict__ xw,
-                                          const float* __restrict__ uv, const Intr& K, double* out) {
+                                          const float* __restrict__ uv, const Intr& K, int kind, double a,
+                                          double* out) {
   double acc[NRED];
 #pragma unroll
   for (int i = 0; i < NRED; i++) acc[i] = 0.0;
@@ -38,6 +40,8 @@ __device__ __forceinline__ void pose_pass(PoseShared& sm, int b, int n, const fl
     if (LIN) {
       double r[2], Jc[12];
       obs_eval<true, false>(sm.rot[b], t, X, K, u, v, r, Jc, nullptr);
+      double rho = 0.0;
+      if (ROBUST) rho = robust_correct(kind, a, r, Jc, nullptr);
       int k = 0;
 #pragma unroll
       for (int a = 0; a < 6; a++) {
@@ -45,9 +49,16 @@ __device__ __forceinline__ void pose_pass(PoseShared& sm, int b, int n, const fl
         for (int c = a; c < 6; c++) acc[k++] += Jc[a] * Jc[c] + Jc[6 + a] * Jc[6 + c];
         acc[21 + a] += Jc[a] * r[0] + Jc[6 + a] * r[1];
       }
-      acc[27] += r[0] * r[0] + r[1] * r[1];
+      acc[27] += ROBUST ? rho : r[0] * r[0] + r[1] * r[1];
     } else {
-      acc[27] += obs_cost(sm.rot[b], t, X, K, u, v);
+      const double s = obs_cost(sm.rot[b], t, X, K, u, v);
+      if (ROBUST) {
+        double rho, rho1;
+        loss_eval(kind, a, s, rho, rho1);
+        acc[27] += rho;
+      } else {
+        acc[27] += s;
+      }
     }
   }
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -69,9 +80,12 @@ __device__ __forceinline__ void pose_pass(PoseShared& sm, int b, int n, const fl
 
 __device__ __forceinline__ int uidx(int a, int b) { return a * 6 - (a * (a - 1)) / 2 + (b - a); }
 
+// ROBUST = false: plain least squares (the reference); true: the loss (kind, a), LORB_LOSS_*
+template <bool ROBUST>
 __global__ void __launch_bounds__(POSE_THREADS)
     pose_only_kernel(int n, const float* __restrict__ xw, const float* __restrict__ uv, Intr K,
-                     double* __restrict__ rt, lorb_ba_options opt, lorb_ba_summary* __restrict__ sum) {
+                     double* __restrict__ rt, lorb_ba_options opt, lorb_ba_summary* __restrict__ sum, int kind,
+                     double a) {
   __shared__ PoseShared sm;
   __shared__ double lin[NRED];
   const int tid = threadIdx.x;
@@ -84,7 +98,7 @@ __global__ void __launch_bounds__(POSE_THREADS)
   __syncthreads();
   if (tid == 0) cam_rotation(sm.x[0], sm.rot[0], true);
   __syncthreads();
-  pose_pass<true>(sm, 0, n, xw, uv, K, lin);
+  pose_pass<true, ROBUST>(sm, 0, n, xw, uv, K, kind, a, lin);
   if (tid == 0) {
     double gm = 0, xn = 0;
     for (int a = 0; a < 21; a++) sm.H[a] = lin[a];
@@ -168,7 +182,7 @@ __global__ void __launch_bounds__(POSE_THREADS)
       cam_rotation(sm.x[cur ^ 1], sm.rot[cur ^ 1], true);
     }
     __syncthreads();
-    pose_pass<false>(sm, cur ^ 1, n, xw, uv, K, lin);
+    pose_pass<false, ROBUST>(sm, cur ^ 1, n, xw, uv, K, kind, a, lin);
     int accepted = 0;
     if (tid == 0) {
       st.acc_cost2 = lin[27];
@@ -178,7 +192,7 @@ __global__ void __launch_bounds__(POSE_THREADS)
     }
     __syncthreads();
     if (st.pad) {  // HandleSuccessfulStep: relinearise, gradient tolerance
-      pose_pass<true>(sm, st.cur, n, xw, uv, K, lin);
+      pose_pass<true, ROBUST>(sm, st.cur, n, xw, uv, K, kind, a, lin);
       if (tid == 0) {
         double gm = 0;
         for (int a = 0; a < 21; a++) sm.H[a] = lin[a];
@@ -240,8 +254,10 @@ extern "C" int lorb_ba_pose_only(lorb_ctx* c, int n, const float* xw, const floa
   Kd.fv = (double)K[0];  // PoseCost projects v with fx (reference src/bundle_adjust.cpp:51)
   Kd.cx = (double)K[2];
   Kd.cy = (double)K[3];
-  LORB_LAUNCH(c, pose_only_kernel, 1, POSE_THREADS, 0, n, (const float*)d, (const float*)(d + b_xw),
-              Kd, (double*)dout, *opt, (lorb_ba_summary*)(dout + 64));
+  const lorb_ba_loss loss = c->ba_loss;
+  LORB_LAUNCH(c, (loss.kind != LORB_LOSS_TRIVIAL ? pose_only_kernel<true> : pose_only_kernel<false>), 1,
+              POSE_THREADS, 0, n, (const float*)d, (const float*)(d + b_xw), Kd, (double*)dout, *opt,
+              (lorb_ba_summary*)(dout + 64), loss.kind, loss.scale);
   LORB_CUDA_TRY(cudaMemcpyAsync(c->h[1].p, dout, down, cudaMemcpyDeviceToHost, c->stream));
   LORB_CUDA_TRY(cudaStreamSynchronize(c->stream));
   memcpy(rt, c->h[1].p, 48);

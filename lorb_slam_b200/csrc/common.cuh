@@ -75,6 +75,7 @@ struct lorb_ctx {
   int chol_coop_blocks = -1;           // same for the dataflow Cholesky (ba_local.cu); 0 = not available
   int chol_chain_blocks = 0;           // and for its chain form
   lorb::Dist* dist = nullptr;
+  lorb_ba_loss ba_loss = {LORB_LOSS_TRIVIAL, 0, 1.0};  // robust loss of every BA solve on this ctx
   void* ba_cache = nullptr;  // reusable lorb_ba_problem of the host-buffer BA calls (ba_local.cu)
   cudaStream_t ba_stream2 = nullptr;  // side branch of the large-path build pass (camera rows beside the Schur pairs)
   cudaEvent_t ba_ev[2] = {nullptr, nullptr};

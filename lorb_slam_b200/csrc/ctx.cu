@@ -2,6 +2,7 @@
 // micro-benchmark (roofline denominator for the matching kernels).
 #include <stdarg.h>
 
+#include <cmath>
 #include <new>
 #include <vector>
 
@@ -293,6 +294,26 @@ void lorb_ba_default_options(lorb_ba_options* o) {
   o->min_relative_decrease = 1e-3;
   o->min_lm_diagonal = 1e-6;
   o->max_lm_diagonal = 1e32;
+}
+
+int lorb_ba_set_loss(lorb_ctx* c, const lorb_ba_loss* loss) {
+  LORB_REQUIRE(c, "ctx");
+  lorb_ba_loss l = {LORB_LOSS_TRIVIAL, 0, 1.0};
+  if (loss) {
+    LORB_REQUIRE(loss->kind >= LORB_LOSS_TRIVIAL && loss->kind <= LORB_LOSS_CAUCHY, "loss kind");
+    LORB_REQUIRE(loss->kind == LORB_LOSS_TRIVIAL || (std::isfinite(loss->scale) && loss->scale > 0.0),
+                 "loss scale must be finite and > 0");
+    l.kind = loss->kind;
+    l.scale = loss->kind == LORB_LOSS_TRIVIAL ? 1.0 : loss->scale;
+  }
+  c->ba_loss = l;
+  return LORB_OK;
+}
+
+int lorb_ba_get_loss(lorb_ctx* c, lorb_ba_loss* loss) {
+  LORB_REQUIRE(c && loss, "ctx / loss");
+  *loss = c->ba_loss;
+  return LORB_OK;
 }
 
 int lorb_microbench_popc(lorb_ctx* c, int kind, int iters, double* words_per_s) {
