@@ -1472,14 +1472,6 @@ __global__ void __launch_bounds__(NB * NB / 4)
   }
 }
 
-// ---- dataflow tiled Cholesky (n > 96, one window): ONE cooperative launch.
-// Lower-triangular 32x32 tiles are numbered column-major and dealt round-robin to
-// co-resident CTAs; a CTA handles its tiles in increasing order.  Tile (i,j) is
-// computed left-looking: A_ij -= sum_{k<j} L_ik L_jk^T as soon as the two source
-// tiles are flagged ready, then POTRF (i == j) or TRSM against L_jj, then its own
-// ready flag.  Every dependency of a tile has a smaller number, so the smallest
-// unfinished tile can always proceed: no deadlock while all CTAs are resident
-// (cooperative launch guarantees that).  Replaces 2 launches per block column.
 // 32x32 POTRF by ONE warp with the tile in registers (lane = row, fully unrolled): per column one
 // broadcast of the pivot, rsqrt, and 31-c shuffle + FMA pairs; no barriers.  The 256-thread
 // shared-memory version took 11.3 us per tile on the critical path of the dataflow factorisation
@@ -1538,153 +1530,15 @@ __device__ __forceinline__ void flag_wait(const int* flag) {
   __syncthreads();
 }
 
-__global__ void __launch_bounds__(256)
-    ba_chol_dataflow_kernel(const BADev* __restrict__ probs, int* __restrict__ flags, int* __restrict__ yflag, int T) {
-  const BADev p = probs[0];
-  LMState* st = p.st;
-  if (st->done) return;
-  __shared__ double A[NB][NB + 1];   // source tile L_ik, then the tile being finished
-  __shared__ double B[NB][NB + 1];   // source tile L_jk, then L_jj (transposed-slot form)
-  __shared__ double idg[NB];
-  __shared__ double sk[NB], vec[NB];  // diagonal tiles: running right-hand side b_j - sum L_jk y_k, and y_k
-  __shared__ int s_ok;
-  const int n = p.n, tid = threadIdx.x;
-  const int ty = tid >> 4, tx = tid & 15;
-  const int n_tiles = T * (T + 1) / 2;
-  if (tid == 0) s_ok = 1;
-  int j = 0, col_start = 0;  // column of the current tile and the number of its first tile
-  for (int t = blockIdx.x; t < n_tiles; t += gridDim.x) {
-    while (t >= col_start + (T - j)) {
-      col_start += T - j;
-      j++;
-    }
-    const int i = j + (t - col_start);
-    const int i0 = i * NB, j0 = j * NB;
-    // diagonal tiles: warp 1 carries the forward substitution (its lane r owns row r of b_j - sum L_jk y_k)
-    const bool ywarp = (i == j) && (tid >> 5) == 1;
-    double skreg = (ywarp && i0 + (tid & 31) < n) ? __ldcg(&p.rhs[i0 + (tid & 31)]) : 0.0, yreg = 0.0;
-    // this thread's 2x2 patch of the tile
-    double acc[2][2];
-#pragma unroll
-    for (int a = 0; a < 2; a++)
-#pragma unroll
-      for (int b = 0; b < 2; b++) {
-        const int r = i0 + 2 * ty + a, c = j0 + 2 * tx + b;
-        acc[a][b] = (r < n && c < n) ? __ldcg(&p.S[(size_t)r * n + c]) : (r == c ? 1.0 : 0.0);
-      }
-    for (int k = 0; k < j; k++) {
-      flag_wait(&flags[i * T + k]);
-      if (i != j) flag_wait(&flags[j * T + k]);
-      const int k0 = k * NB;
-      if (ywarp) {  // y_k was published right after POTRF(k): normally no wait; its load overlaps the tile loads
-        if ((tid & 31) == 0) {
-          while (*reinterpret_cast<const volatile int*>(&yflag[k]) == 0) {
-          }
-          __threadfence();
-        }
-        __syncwarp();
-        yreg = __ldcg(&p.rhs[k0 + (tid & 31)]);
-      }
-      {
-        // both source tiles in flight at once (8 independent loads per thread), then to shared memory
-        double ta[4], tb[4];
-#pragma unroll
-        for (int q = 0; q < 4; q++) {
-          const int e = tid + 256 * q, r = e >> 5, c = e & 31;
-          ta[q] = (i0 + r < n) ? __ldcg(&p.S[(size_t)(i0 + r) * n + k0 + c]) : 0.0;
-          tb[q] = (j0 + r < n) ? __ldcg(&p.S[(size_t)(j0 + r) * n + k0 + c]) : 0.0;
-        }
-#pragma unroll
-        for (int q = 0; q < 4; q++) {
-          const int e = tid + 256 * q, r = e >> 5, c = e & 31;
-          A[r][c] = ta[q];
-          B[r][c] = tb[q];
-        }
-      }
-      __syncthreads();
-      if (ywarp) {
-        vec[tid & 31] = yreg;
-        __syncwarp();
-        double a2 = 0;
-#pragma unroll 8
-        for (int m = 0; m < NB; m++) a2 += A[tid & 31][m] * vec[m];
-        skreg -= a2;
-        __syncwarp();
-      }
-#pragma unroll 8
-      for (int m = 0; m < NB; m++) {
-        const double a0 = A[2 * ty][m], a1 = A[2 * ty + 1][m];
-        const double b0 = B[2 * tx][m], b1 = B[2 * tx + 1][m];
-        acc[0][0] -= a0 * b0;
-        acc[0][1] -= a0 * b1;
-        acc[1][0] -= a1 * b0;
-        acc[1][1] -= a1 * b1;
-      }
-      __syncthreads();
-    }
-#pragma unroll
-    for (int a = 0; a < 2; a++)
-#pragma unroll
-      for (int b = 0; b < 2; b++) A[2 * ty + a][2 * tx + b] = acc[a][b];
-    if (ywarp) sk[tid & 31] = skreg;
-    __syncthreads();
-    if (i == j) {
-      // POTRF: warp 0, tile in registers; L_rc (r>c) comes back at A[c][r]
-      if (tid < 32) potrf32_warp(A, idg, &s_ok, tid);
-      __syncthreads();
-      for (int e = tid; e < NB * NB; e += 256) {
-        const int r = e >> 5, c = e & 31;
-        if (i0 + r < n && c < r) p.S[(size_t)(i0 + r) * n + j0 + c] = A[c][r];
-      }
-      if (tid < NB) {
-        if (i0 + tid < n) p.S[(size_t)(i0 + tid) * n + j0 + tid] = 1.0 / idg[tid];
-        p.dinv[(size_t)j * NB + tid] = idg[tid];
-      }
-    } else {
-      flag_wait(&flags[j * T + j]);
-      for (int e = tid; e < NB * NB; e += 256) {
-        const int r = e >> 5, c = e & 31;  // B[m][c] = L_cm for m < c
-        B[c][r] = (r > c && j0 + r < n) ? __ldcg(&p.S[(size_t)(j0 + r) * n + j0 + c]) : 0.0;
-      }
-      if (tid < NB) idg[tid] = __ldcg(&p.dinv[(size_t)j * NB + tid]);
-      __syncthreads();
-      if (tid < 32) trsm32_warp(A, B, idg, tid);
-      __syncthreads();
-      for (int e = tid; e < NB * NB; e += 256) {
-        const int r = e >> 5, c = e & 31;
-        if (i0 + r < n && j0 + c < n) p.S[(size_t)(i0 + r) * n + j0 + c] = A[r][c];
-      }
-    }
-    __threadfence();  // every thread publishes its part of the tile before the flag goes up
-    __syncthreads();
-    if (tid == 0) atomicExch(&flags[i * T + j], 1);
-    if (i == j && tid < 32) {
-      // L_jj y_j = b_j - sum_k L_jk y_k (off the factorisation's critical path: L_jj is already out).
-      // L_rc (r > c) sits at A[c][r], idg[c] = 1 / L_cc.
-      double v = sk[tid];
-#pragma unroll 8
-      for (int c = 0; c < NB; c++) {
-        const double yc = __shfl_sync(0xffffffffu, v, c) * idg[c];
-        if (tid == c) v = yc;
-        if (tid > c) v -= A[c][tid] * yc;
-      }
-      if (i0 + tid < n) p.rhs[i0 + tid] = v;
-      __threadfence();
-      __syncwarp();
-      if (tid == 0) atomicExch(&yflag[j], 1);
-    }
-  }
-  __syncthreads();
-  if (tid == 0 && !s_ok) st->solve_ok = 0;
-}
-
-// ---- dataflow tiled Cholesky, chain form (n > 96, one window): ONE cooperative launch.
+// ---- dataflow tiled Cholesky, chain form (n > 143, one window): ONE cooperative launch.
 // The factorisation's critical path is POTRF(j) -> TRSM(j+1, j) -> last update of (j+1, j+1) ->
-// POTRF(j+1).  In ba_chol_dataflow_kernel those three steps belong to three different CTAs, so a
-// block column costs two publish / consume hops through global memory and two tile reloads on top
-// of the arithmetic.  Here CTA 0 walks the whole chain with L_jj and L_(j+1)j staying in its shared
-// memory, and every other CTA is a helper working through a list of items in column order:
-//   * normal tiles (i, j), i >= j + 2: left-looking accumulation, TRSM against L_jj (as before);
+// POTRF(j+1).  With 32x32 tiles dealt round-robin to CTAs those three steps belong to three
+// different CTAs, so a block column costs two publish / consume hops through global memory and two
+// tile reloads on top of the arithmetic.  Here CTA 0 walks the whole chain with L_jj and L_(j+1)j
+// staying in its shared memory, and every other CTA is a helper working through a list of items in
+// column order:
+//   * normal tiles (i, j), i >= j + 2: left-looking accumulation A_ij -= sum_{k<j} L_ik L_jk^T as
+//     soon as both source tiles are flagged ready, then TRSM against L_jj;
 //   * the "sub partial" of column j: S(j+1, j) - sum_{k<j} L(j+1, k) L(j, k)^T, left in place for
 //     the chain CTA, which only has to apply L_jj^-T;
 //   * the "diagonal partial" of block d = j + 1: S(d, d) - sum_{k<=d-2} L(d, k) L(d, k)^T and the
@@ -1720,12 +1574,14 @@ __global__ void __launch_bounds__(256)
     // ================= the chain
     __shared__ double Dn[NB][NB + 1];  // next diagonal partial, fetched by idle warps during POTRF
     __shared__ double skn[NB];
-    __shared__ int have_next;
+    __shared__ int have_next;  // halves of Dn fetched: warp 2 rows 0-15 and skn, warp 3 rows 16-31
     if (tid == 0) have_next = 0;
     __syncthreads();
     for (int j = 0; j < T; j++) {
       const int j0 = j * NB, s0 = (j + 1) * NB;
-      const bool pre = have_next != 0;  // uniform: written before the last barrier of the previous column
+      // uniform: written before the last barrier of the previous column.  Warps 2 and 3 read the
+      // partial's flag each on their own, so the prefetched tile is complete only when both counted in.
+      const bool pre = have_next == 2;
       if (j >= 2 && !pre) flag_wait(&dflag[j]);
       // diagonal tile (partial) minus this CTA's own last term X X^T (X = L_j(j-1), still in X)
       double acc[2][2];
@@ -1798,7 +1654,7 @@ __global__ void __launch_bounds__(256)
             }
             if (warp == 2)
               skn[lane] = jn0 + lane < n ? (jn >= 2 ? __ldcg(&ypart[jn * NB + lane]) : __ldcg(&p.rhs[jn0 + lane])) : 0.0;
-            if (warp == 3 && lane == 0) have_next = 1;
+            if (lane == 0) atomicAdd(&have_next, 1);
           }
         }
       } else if (sub && warp >= 4) {
@@ -2015,7 +1871,7 @@ __global__ void __launch_bounds__(256)
     idg[tid] = __ldcg(&p.dinv[(size_t)k * NB + tid]);
   }
   load_tile(2, k, k);
-  // ---------------- forward: L y = b (already done inside ba_chol_dataflow_kernel when fwd_done)
+  // ---------------- forward: L y = b (already done inside ba_chol_chain_kernel when fwd_done)
   if (!fwd_done && k > 0) load_tile(0, k, 0);
   __syncthreads();
   for (int j = 0; j < (fwd_done ? 0 : k); j++) {
@@ -3134,45 +2990,27 @@ static int run_cholesky(lorb_ba_problem* pb) {
     return LORB_OK;
   }
   const int nblk = (n + NB - 1) / NB;
-  if (c->chol_coop_blocks < 0) {  // per context (= per device and calling thread)
-    int dev_coop = 0, per_sm = 0;
-    cudaDeviceGetAttribute(&dev_coop, cudaDevAttrCooperativeLaunch, c->device);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ba_chol_dataflow_kernel, 256, 0);
-    const char* e = getenv("LORB_CHOL_DATAFLOW");
-    c->chol_coop_blocks = (dev_coop && per_sm > 0 && !(e && atoi(e) == 0)) ? per_sm * c->sm_count : 0;
-    int per_sm2 = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm2, ba_chol_chain_kernel, 256, 0);
-    c->chol_chain_blocks = per_sm2 * c->sm_count;
+  if (c->chol_chain_blocks < 0) {  // per context (= per device and calling thread)
+    int per_sm = 0;
+    LORB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ba_chol_chain_kernel, 256, 0));
+    c->chol_chain_blocks = per_sm * c->sm_count;
   }
-  const int coop_blocks = c->chol_coop_blocks;
-  const bool coop_ok = coop_blocks > 0;
-  // (one CTA per block row of the solve must be co-resident as well)
-  if (coop_ok && nw == 1 && nblk <= c->sm_count) {
+  // one window, one CTA per block row of the solve co-resident, and at least one helper beside the chain CTA
+  if (nw == 1 && nblk <= c->sm_count && c->chol_chain_blocks >= 2) {
     const int n_tiles = nblk * (nblk + 1) / 2;
-    // tile flags [T*T], y / x flags [2T], partial flags [2T] (chain form), forward-substitution partials [T][32]
+    // tile flags [T*T], y / x flags [2T], partial flags [2T], forward-substitution partials [T][32]
     const size_t flag_ints = (size_t)nblk * nblk + 4 * (size_t)nblk + 2;
     LORB_TRY(dev_reserve(c, 14, flag_ints * 4 + (size_t)nblk * NB * 8));
     int* flags = c->d[14].as<int>();
     LORB_CUDA_TRY(cudaMemsetAsync(flags, 0, flag_ints * 4, c->stream));
     int T = nblk;
     int* sflags = flags + (size_t)nblk * nblk;  // y flags [T], x flags [T]
-    static const int chain_env = [] {
-      const char* e = getenv("LORB_CHOL_CHAIN");  // 0: the round-robin dataflow kernel (no dedicated chain CTA)
-      return e ? atoi(e) : 1;
-    }();
-    if (chain_env) {
-      int* pflag = sflags + 2 * (size_t)nblk;
-      double* ypart = reinterpret_cast<double*>(flags + (((size_t)nblk * nblk + 4 * (size_t)nblk + 1) & ~(size_t)1));
-      void* cargs[] = {(void*)&dp, (void*)&flags, (void*)&sflags, (void*)&pflag, (void*)&ypart, (void*)&T};
-      LORB_CUDA_TRY(cudaLaunchCooperativeKernel((void*)ba_chol_chain_kernel,
-                                                dim3(std::min(n_tiles + 1, c->chol_chain_blocks)), dim3(256), cargs, 0,
-                                                c->stream));
-    } else {
-      void* args[] = {(void*)&dp, (void*)&flags, (void*)&sflags, (void*)&T};
-      LORB_CUDA_TRY(cudaLaunchCooperativeKernel((void*)ba_chol_dataflow_kernel,
-                                                dim3(std::min(n_tiles, coop_blocks)), dim3(256), args, 0,
-                                                c->stream));
-    }
+    int* pflag = sflags + 2 * (size_t)nblk;
+    double* ypart = reinterpret_cast<double*>(flags + (((size_t)nblk * nblk + 4 * (size_t)nblk + 1) & ~(size_t)1));
+    void* cargs[] = {(void*)&dp, (void*)&flags, (void*)&sflags, (void*)&pflag, (void*)&ypart, (void*)&T};
+    LORB_CUDA_TRY(cudaLaunchCooperativeKernel((void*)ba_chol_chain_kernel,
+                                              dim3(std::min(n_tiles + 1, c->chol_chain_blocks)), dim3(256), cargs, 0,
+                                              c->stream));
     c->launches++;
     int fwd_done = 1;  // the factorisation kernel also ran the forward substitution
     void* args2[] = {(void*)&dp, (void*)&sflags, (void*)&T, (void*)&fwd_done};
@@ -3180,12 +3018,11 @@ static int run_cholesky(lorb_ba_problem* pb) {
                                               dim3(256), args2, 0, c->stream));
     c->launches++;
     return LORB_OK;
-  } else {
-    for (int kb = 0; kb < nblk; kb++) {
-      LORB_LAUNCH(c, ba_chol_panel_kernel, dim3(nblk - kb, nw), NB * NB / 4, 0, dp, kb);
-      const int m = nblk - kb - 1;
-      if (m > 0) LORB_LAUNCH(c, ba_chol_update_kernel, dim3(m * (m + 1) / 2, nw), 256, 0, dp, kb, nblk);
-    }
+  }
+  for (int kb = 0; kb < nblk; kb++) {
+    LORB_LAUNCH(c, ba_chol_panel_kernel, dim3(nblk - kb, nw), NB * NB / 4, 0, dp, kb);
+    const int m = nblk - kb - 1;
+    if (m > 0) LORB_LAUNCH(c, ba_chol_update_kernel, dim3(m * (m + 1) / 2, nw), 256, 0, dp, kb, nblk);
   }
   LORB_REQUIRE((size_t)n * 8 <= 200 * 1024, "reduced camera system too large for the solve kernel");
   LORB_CUDA_TRY(cudaFuncSetAttribute(ba_chol_solve_kernel,

@@ -72,8 +72,7 @@ struct lorb_ctx {
   std::vector<long long> tc_chunk_units;  // first unit of every <= 16384-pair chunk of the plan (+ end)
   size_t tc_keys_rows = 0;
   int proj_coop_blocks[2] = {-1, -1};  // co-resident CTAs of the cooperative claim resolution (match_proj.cu)
-  int chol_coop_blocks = -1;           // same for the dataflow Cholesky (ba_local.cu); 0 = not available
-  int chol_chain_blocks = 0;           // and for its chain form
+  int chol_chain_blocks = -1;          // same for the chain Cholesky (ba_local.cu); -1 = not yet queried
   lorb::Dist* dist = nullptr;
   lorb_ba_loss ba_loss = {LORB_LOSS_TRIVIAL, 0, 1.0};  // robust loss of every BA solve on this ctx
   void* ba_cache = nullptr;  // reusable lorb_ba_problem of the host-buffer BA calls (ba_local.cu)
@@ -204,12 +203,6 @@ __device__ __forceinline__ uint32_t hamming256_csa(const uint32_t (&q)[8], const
   uint32_t ones = imad((uint32_t)__popc(s3), 1u, (uint32_t)__popc(x7));
   uint32_t d = imad((uint32_t)__popc(tw), 2u, ones);
   return imad((uint32_t)__popc(fo), 4u, d);
-}
-
-template <bool CSA>
-__device__ __forceinline__ uint32_t hamming256(const uint32_t (&q)[8], const uint32_t (&t)[8]) {
-  if (CSA) return hamming256_csa(q, t);
-  return hamming256_popc8(q, t);
 }
 
 // Packed (distance, index) keys: distance in the high bits, index in the low

@@ -67,7 +67,7 @@ __global__ void __launch_bounds__(256) popc_bench_kernel(uint32_t* sink, int ite
     for (int i = 0; i < 8; i++) t[i] = t[i] * 1664525u + 1013904223u;  // 8 IMAD per 4 pairs
 #pragma unroll
     for (int k = 0; k < 4; k++) {
-      uint32_t d = hamming256<CSA>(q[k], t);
+      uint32_t d = CSA ? hamming256_csa(q[k], t) : hamming256_popc8(q[k], t);
       best[k] = min(best[k], make_key(d, (uint32_t)it));
     }
   }
@@ -233,6 +233,11 @@ int lorb_ctx_create(int device, lorb_ctx** out) {
   if (prop.major != 10) {
     set_error("device %d is sm_%d%d; this library is built for sm_100a only", device, prop.major,
               prop.minor);
+    delete c;
+    return LORB_ERR_CUDA;
+  }
+  if (!prop.cooperativeLaunch) {  // the claim resolution and the single-window Cholesky are cooperative launches
+    set_error("device %d does not support cooperative launch, which this library needs", device);
     delete c;
     return LORB_ERR_CUDA;
   }

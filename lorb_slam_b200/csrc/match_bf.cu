@@ -36,7 +36,7 @@ constexpr int TILE_CHUNK = 256;  // trains per shared-memory stage (8 KB)
 //   rowkey2[k]  running second min                               [MODE 1]
 //   colkey      shared array, entry j = min over queries of
 //               (dist<<20 | query index) for train j             [MODE 0]
-template <int QPT, bool CSA, int MODE>
+template <int QPT, int MODE>
 __device__ __forceinline__ void scan_trains(const uint4* __restrict__ Bs, int nt, uint32_t t_base,
                                             const uint32_t (&q)[QPT][8], const uint32_t (&qidx)[QPT],
                                             uint32_t (&rowkey)[QPT], uint32_t (&rowkey2)[QPT],
@@ -52,7 +52,7 @@ __device__ __forceinline__ void scan_trains(const uint4* __restrict__ Bs, int nt
       uint32_t ck = KEY_NONE;
 #pragma unroll
       for (int k = 0; k < QPT; k++) {
-        const uint32_t d = hamming256<CSA>(q[k], tw);
+        const uint32_t d = hamming256_csa(q[k], tw);
         const uint32_t rk = make_key(d, t_base + (uint32_t)t);
         if (MODE == 1) {
           rowkey2[k] = min(rowkey2[k], max(rowkey[k], rk));
@@ -93,7 +93,7 @@ __device__ __forceinline__ void load_queries(const uint4* __restrict__ Q, int nq
 // grid = (query tiles, train splits).  MODE 0: cross-check keys into
 // fwd_key[nq] / bwd_key[nt] (global atomicMin).  MODE 1: per split best/second
 // row keys into part[split][nq][2].
-template <int QPT, bool CSA, int MODE>
+template <int QPT, int MODE>
 __global__ void __launch_bounds__(TILE_THREADS)
     hamming_tile_kernel(const uint4* __restrict__ Q, int nq, const uint4* __restrict__ T, int nt,
                         int trains_per_split, uint32_t* __restrict__ fwd_key,
@@ -135,8 +135,7 @@ __global__ void __launch_bounds__(TILE_THREADS)
       __syncthreads();
     }
     mbar_wait(&bar[c & 1], (uint32_t)((c >> 1) & 1));
-    scan_trains<QPT, CSA, MODE>(&Bs[c & 1][0], len, (uint32_t)c0, q, qidx, rowkey, rowkey2, colkey,
-                                lane);
+    scan_trains<QPT, MODE>(&Bs[c & 1][0], len, (uint32_t)c0, q, qidx, rowkey, rowkey2, colkey, lane);
     __syncthreads();
     if (MODE == 0) {
       for (int j = tid; j < len; j += TILE_THREADS)
@@ -350,7 +349,7 @@ __global__ void __launch_bounds__(128)
 // ------------------------------------------------------------------ sweep
 constexpr int SWEEP_THREADS = 512;
 
-template <int QPT, bool CSA>
+template <int QPT>
 __global__ void __launch_bounds__(SWEEP_THREADS, 1)
     sweep_kernel(const uint4* __restrict__ bank, const uint4* __restrict__ bank_b, int n_desc,
                  const int2* __restrict__ pairs, int n_pairs,
@@ -421,7 +420,7 @@ __global__ void __launch_bounds__(SWEEP_THREADS, 1)
 #pragma unroll
     for (int k = 0; k < QPT; k++) rowkey[k] = rowkey2[k] = KEY_NONE;
     mbar_wait(&bar[1 + (i & 1)], (uint32_t)((i >> 1) & 1));
-    scan_trains<QPT, CSA, 0>(Bs, n_desc, 0u, q, qidx, rowkey, rowkey2, colkey, lane);
+    scan_trains<QPT, 0>(Bs, n_desc, 0u, q, qidx, rowkey, rowkey2, colkey, lane);
     __syncthreads();  // all column keys final
     // mutual test + minDist + max(2*minDist,30) filter (reference :42-56)
     int cnt = 0, lmin = 1 << 30;
@@ -481,33 +480,13 @@ static size_t sweep_smem_bytes(int n_desc) {
   return 3 * buf + (size_t)((n_desc + 31) & ~31) * 4 + 4 * 8 + 40 * 4;
 }
 
-// 0 = plain 8-popc body, 1 = carry-save body.  Default picked from the
-// measured micro-benchmark (profiles/); override with LORB_HAMMING_CSA=0/1.
-static bool use_csa() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("LORB_HAMMING_CSA");
-    v = e ? (atoi(e) != 0) : 1;
-  }
-  return v != 0;
-}
-
 template <int QPT>
 static int launch_sweep_qpt(lorb_ctx* c, const uint4* bank, const uint4* bank_b, int n_desc,
                             const int2* pairs, int n_pairs, int* out) {
   const size_t smem = sweep_smem_bytes(n_desc);
   const int grid = std::min(n_pairs, c->sm_count);
-  if (use_csa()) {
-    LORB_CUDA_TRY(cudaFuncSetAttribute(sweep_kernel<QPT, true>,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    LORB_LAUNCH(c, (sweep_kernel<QPT, true>), grid, SWEEP_THREADS, smem, bank, bank_b, n_desc, pairs,
-                n_pairs, out);
-  } else {
-    LORB_CUDA_TRY(cudaFuncSetAttribute(sweep_kernel<QPT, false>,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    LORB_LAUNCH(c, (sweep_kernel<QPT, false>), grid, SWEEP_THREADS, smem, bank, bank_b, n_desc, pairs,
-                n_pairs, out);
-  }
+  LORB_CUDA_TRY(cudaFuncSetAttribute(sweep_kernel<QPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  LORB_LAUNCH(c, sweep_kernel<QPT>, grid, SWEEP_THREADS, smem, bank, bank_b, n_desc, pairs, n_pairs, out);
   return LORB_OK;
 }
 
@@ -541,16 +520,10 @@ static int launch_tiles(lorb_ctx* c, const uint4* dq, int nq, const uint4* dt, i
   splits = (nt + per - 1) / per;
   if (n_splits_out) *n_splits_out = splits;
   dim3 grid(q_tiles, splits);
-  const bool csa = use_csa();
-#define LORB_TILE(QPT_, CSA_)                                                                   \
-  LORB_LAUNCH(c, (hamming_tile_kernel<QPT_, CSA_, MODE>), grid, TILE_THREADS, 0, dq, nq, dt, nt, \
-              per, fwd, bwd, part)
-  if (wide) {
-    if (csa) LORB_TILE(4, true); else LORB_TILE(4, false);
-  } else {
-    if (csa) LORB_TILE(1, true); else LORB_TILE(1, false);
-  }
-#undef LORB_TILE
+  if (wide)
+    LORB_LAUNCH(c, (hamming_tile_kernel<4, MODE>), grid, TILE_THREADS, 0, dq, nq, dt, nt, per, fwd, bwd, part);
+  else
+    LORB_LAUNCH(c, (hamming_tile_kernel<1, MODE>), grid, TILE_THREADS, 0, dq, nq, dt, nt, per, fwd, bwd, part);
   return LORB_OK;
 }
 

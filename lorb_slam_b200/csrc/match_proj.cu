@@ -13,7 +13,7 @@
 //                            reference's iteration order (cell column major),
 //                            level / window / stereo gates, Hamming distance;
 //                            ordered candidate lists (kp | dist<<20) in a CSR
-//   3. resolve_kernel        one CTA: the claim semantics as a monotone
+//   3. resolve_coop_kernel   one cooperative launch: the claim semantics as a monotone
 //                            fixpoint — fp[kp] = order index of the first
 //                            protecting point that took kp; point k ignores
 //                            candidates with fp[kp] < k.  Every fixpoint equals
@@ -427,143 +427,6 @@ __device__ __forceinline__ int choose_warp(const uint32_t* __restrict__ cand, in
   return bestIdx;
 }
 
-// SMEM = true: the two claim arrays and the octaves live in shared memory
-// (12 B per keypoint), so the per-candidate dependent loads cost ~30 cycles
-// instead of an L2 round trip; used whenever they fit.
-template <int MODE, bool SMEM>
-__global__ void __launch_bounds__(1024)
-    resolve_kernel(int n_kp, int n_pts, const int* __restrict__ claim_obs,
-                   const int* __restrict__ kp_octave, const float* __restrict__ kp_angle,
-                   const int* __restrict__ mp_nobs, const float* __restrict__ last_angle,
-                   const int* __restrict__ seg_start, const int* __restrict__ seg_len,
-                   const uint32_t* __restrict__ cand, int* __restrict__ fp_a, int* __restrict__ fp_b,
-                   int* __restrict__ choice, int* __restrict__ out_for_kp, int* __restrict__ res,
-                   const unsigned long long* __restrict__ cand_total, unsigned long long cand_cap) {
-  // the candidate arena overflowed: the segments point past its end and the host repeats the
-  // search with the exact size -- nothing to resolve in this attempt
-  if (*cand_total > cand_cap) return;
-  __shared__ int s_changed, s_count;
-  __shared__ int s_hist[LORB_HISTO_LENGTH];
-  __shared__ int s_ind[3];
-  extern __shared__ int s_dyn[];
-  const int tid = threadIdx.x;
-  const int INF = 0x7fffffff;
-  if (SMEM) {
-    fp_a = s_dyn;
-    fp_b = s_dyn + n_kp;
-    int* oct = s_dyn + 2 * n_kp;
-    for (int i = tid; i < n_kp; i += blockDim.x) oct[i] = kp_octave[i];
-    kp_octave = oct;
-  }
-  for (int i = tid; i < n_kp; i += blockDim.x) {
-    fp_a[i] = claim_obs[i] > 0 ? -1 : INF;
-    out_for_kp[i] = -1;
-  }
-  for (int k = tid; k < n_pts; k += blockDim.x) choice[k] = -2;  // "not evaluated yet"
-  int* fp_cur = fp_a;
-  int* fp_new = fp_b;
-  int sweeps = 0;
-  for (;;) {
-    if (tid == 0) s_changed = 0;
-    for (int i = tid; i < n_kp; i += blockDim.x) fp_new[i] = claim_obs[i] > 0 ? -1 : INF;
-    __syncthreads();
-    int changed = 0;
-    {
-      // RG lanes per point; the loop is warp-uniform so every lane reaches the shuffles
-      const int lane = tid & (RG - 1), ngroups = blockDim.x / RG, per_warp = 32 / RG;
-      for (int base = (tid >> 5) * per_warp; base < n_pts; base += ngroups) {
-        const int k = base + ((tid & 31) / RG);
-        const int n = k < n_pts ? seg_len[k] : 0;
-        const int c = choose_warp<MODE>(cand, n > 0 ? seg_start[k] : 0, n, fp_cur, k, kp_octave, lane);
-        if (lane == 0 && k < n_pts) {
-          if (c != choice[k]) {
-            choice[k] = c;
-            changed = 1;
-          }
-          if (c >= 0 && mp_nobs[k] > 0) atomicMin(&fp_new[c], k);
-        }
-      }
-    }
-    if (changed) s_changed = 1;
-    __syncthreads();
-    sweeps++;
-    const int any = s_changed;
-    int* t = fp_cur;
-    fp_cur = fp_new;
-    fp_new = t;
-    __syncthreads();
-    if (!any) break;
-  }
-  // final holder of a keypoint = last point that took it
-  if (tid == 0) s_count = 0;
-  if (tid < LORB_HISTO_LENGTH) s_hist[tid] = 0;
-  __syncthreads();
-  int cnt = 0;
-  for (int k = tid; k < n_pts; k += blockDim.x) {
-    const int c = choice[k];
-    if (c >= 0) {
-      cnt++;
-      atomicMax(&out_for_kp[c], k);
-      if (MODE == 1) {
-        float rot = __fsub_rn(last_angle[k], kp_angle[c]);  // :181-188
-        if (rot < 0.0f) rot = __fadd_rn(rot, 360.0f);
-        int bin = (int)roundf(__fmul_rn(rot, (float)LORB_HISTO_LENGTH / 360.0f));
-        if (bin == LORB_HISTO_LENGTH) bin = 0;
-        atomicAdd(&s_hist[bin], 1);
-      }
-    }
-  }
-  if (cnt) atomicAdd(&s_count, cnt);
-  __syncthreads();
-  if (MODE == 1) {
-    if (tid == 0) {  // ComputeThreeMaxima :387-428
-      int max1 = 0, max2 = 0, max3 = 0, i1 = -1, i2 = -1, i3 = -1;
-      for (int i = 0; i < LORB_HISTO_LENGTH; i++) {
-        const int s = s_hist[i];
-        if (s > max1) {
-          max3 = max2; max2 = max1; max1 = s;
-          i3 = i2; i2 = i1; i1 = i;
-        } else if (s > max2) {
-          max3 = max2; max2 = s;
-          i3 = i2; i2 = i;
-        } else if (s > max3) {
-          max3 = s;
-          i3 = i;
-        }
-      }
-      if ((float)max2 < __fmul_rn(0.1f, (float)max1)) {
-        i2 = -1;
-        i3 = -1;
-      } else if ((float)max3 < __fmul_rn(0.1f, (float)max1)) {
-        i3 = -1;
-      }
-      s_ind[0] = i1; s_ind[1] = i2; s_ind[2] = i3;
-    }
-    __syncthreads();
-    int dropped = 0;
-    for (int k = tid; k < n_pts; k += blockDim.x) {
-      const int c = choice[k];
-      if (c >= 0) {
-        float rot = __fsub_rn(last_angle[k], kp_angle[c]);
-        if (rot < 0.0f) rot = __fadd_rn(rot, 360.0f);
-        int bin = (int)roundf(__fmul_rn(rot, (float)LORB_HISTO_LENGTH / 360.0f));
-        if (bin == LORB_HISTO_LENGTH) bin = 0;
-        if (bin != s_ind[0] && bin != s_ind[1] && bin != s_ind[2]) {
-          out_for_kp[c] = -2;  // :204-214 (every entry of a rejected bin NULLs its keypoint)
-          dropped++;
-        }
-      }
-    }
-    __syncthreads();  // all atomicMax above are ordered before these plain stores by the earlier barrier
-    if (dropped) atomicSub(&s_count, dropped);
-  }
-  __syncthreads();
-  if (tid == 0) {
-    res[0] = s_count;
-    res[1] = sweeps;
-  }
-}
-
 // ---- Frame::IsInFrustum + MapPoint::PredictScale, one thread per map point
 struct FrustumDev {
   float tcw[16];
@@ -621,7 +484,7 @@ __global__ void frustum_kernel(FrustumDev F, int n, const float* __restrict__ xw
   vcos[i] = vc;
 }
 
-// ---- 3b. the same claim resolution as one COOPERATIVE multi-CTA launch: the
+// ---- 3b. the claim resolution runs as one COOPERATIVE multi-CTA launch: the
 // per-sweep evaluation is latency-bound (a handful of dependent loads per
 // point), so it is spread over all SMs (8 lanes per point, every point in
 // flight at once) with a grid-wide barrier between the phases of a sweep.
@@ -636,7 +499,9 @@ __global__ void __launch_bounds__(256)
                         int* out_for_kp, int* res, int* scratch,
                         const unsigned long long* __restrict__ cand_total, unsigned long long cand_cap) {
   namespace cg = cooperative_groups;
-  if (*cand_total > cand_cap) return;  // arena overflow (see resolve_kernel): every CTA leaves, before any grid barrier
+  // the candidate arena overflowed: the segments point past its end and the host repeats the search
+  // with the exact size -- nothing to resolve in this attempt; every CTA leaves, before any grid barrier
+  if (*cand_total > cand_cap) return;
   cg::grid_group grid = cg::this_grid();
   const int INF = 0x7fffffff;
   const int gtid = blockIdx.x * blockDim.x + threadIdx.x, gsize = gridDim.x * blockDim.x;
@@ -864,46 +729,32 @@ static int run_search(lorb_ctx* c, const lorb_frame_view* fv, int n_pts, const u
     // per context (= per device and calling thread): co-resident CTAs of the cooperative kernel
     int* coop_blocks = c->proj_coop_blocks;
     if (coop_blocks[MODE] < 0) {
-      int dev_coop = 0, per_sm = 0;
-      cudaDeviceGetAttribute(&dev_coop, cudaDevAttrCooperativeLaunch, c->device);
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, resolve_coop_kernel<MODE>, 256, 0);
-      const char* e = getenv("LORB_RESOLVE_COOP");
-      coop_blocks[MODE] = (dev_coop && per_sm > 0 && !(e && atoi(e) == 0)) ? per_sm * c->sm_count : 0;
-    }
-    if (coop_blocks[MODE] > 0) {
-      int* d_scratch = reinterpret_cast<int*>(wsd + w_scratch);
-      const int want = std::max(1, (int)(((size_t)std::max(n_pts, 1) * RG + 255) / 256));
-      const int grid = std::min(want, coop_blocks[MODE]);
-      int a_nkp = n_kp, a_npts = n_pts;
-      const int* a_claim = f.claim_obs;
-      const int* a_oct = f.octave;
-      const float* a_ang = f.angle;
-      const uint32_t* a_cand = d_cand;
-      const int* a_segs = d_segs;
-      const int* a_segl = d_segl;
-      const unsigned long long* a_total = d_counter;
-      unsigned long long a_cap = cand_cap;
-      void* args[] = {&a_nkp, &a_npts, &a_claim, &a_oct, &a_ang, (void*)&d_nobs, (void*)&d_lang,
-                      &a_segs, &a_segl, &a_cand, &d_fpa, &d_fpb, &d_choice, &d_forkp, &d_res,
-                      &d_scratch, &a_total, &a_cap};
-      LORB_CUDA_TRY(cudaLaunchCooperativeKernel((void*)resolve_coop_kernel<MODE>, dim3(grid),
-                                                dim3(256), args, 0, c->stream));
-      c->launches++;
-    } else {
-      const size_t res_smem = (size_t)n_kp * 12;
-      if (res_smem <= 160 * 1024) {
-        LORB_CUDA_TRY(cudaFuncSetAttribute(resolve_kernel<MODE, true>,
-                                           cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)std::max<size_t>(res_smem, 16)));
-        LORB_LAUNCH(c, (resolve_kernel<MODE, true>), 1, 1024, res_smem, n_kp, n_pts, f.claim_obs,
-                    f.octave, f.angle, d_nobs, d_lang, d_segs, d_segl, d_cand, d_fpa, d_fpb, d_choice,
-                    d_forkp, d_res, d_counter, (unsigned long long)cand_cap);
-      } else {
-        LORB_LAUNCH(c, (resolve_kernel<MODE, false>), 1, 1024, 0, n_kp, n_pts, f.claim_obs, f.octave,
-                    f.angle, d_nobs, d_lang, d_segs, d_segl, d_cand, d_fpa, d_fpb, d_choice, d_forkp,
-                    d_res, d_counter, (unsigned long long)cand_cap);
+      int per_sm = 0;
+      LORB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, resolve_coop_kernel<MODE>, 256, 0));
+      if (per_sm == 0) {
+        set_error("projection search: the claim resolution kernel cannot be resident on this device");
+        return LORB_ERR_STATE;
       }
+      coop_blocks[MODE] = per_sm * c->sm_count;
     }
+    int* d_scratch = reinterpret_cast<int*>(wsd + w_scratch);
+    const int want = std::max(1, (int)(((size_t)std::max(n_pts, 1) * RG + 255) / 256));
+    const int grid = std::min(want, coop_blocks[MODE]);
+    int a_nkp = n_kp, a_npts = n_pts;
+    const int* a_claim = f.claim_obs;
+    const int* a_oct = f.octave;
+    const float* a_ang = f.angle;
+    const uint32_t* a_cand = d_cand;
+    const int* a_segs = d_segs;
+    const int* a_segl = d_segl;
+    const unsigned long long* a_total = d_counter;
+    unsigned long long a_cap = cand_cap;
+    void* args[] = {&a_nkp, &a_npts, &a_claim, &a_oct, &a_ang, (void*)&d_nobs, (void*)&d_lang,
+                    &a_segs, &a_segl, &a_cand, &d_fpa, &d_fpb, &d_choice, &d_forkp, &d_res,
+                    &d_scratch, &a_total, &a_cap};
+    LORB_CUDA_TRY(cudaLaunchCooperativeKernel((void*)resolve_coop_kernel<MODE>, dim3(grid),
+                                              dim3(256), args, 0, c->stream));
+    c->launches++;
     LORB_CUDA_TRY(cudaMemcpyAsync(outd + r_cnt, d_counter, 16, cudaMemcpyDeviceToDevice, c->stream));
     LORB_CUDA_TRY(cudaMemcpyAsync(c->h[1].p, outd, op.off, cudaMemcpyDeviceToHost, c->stream));
     LORB_CUDA_TRY(cudaStreamSynchronize(c->stream));

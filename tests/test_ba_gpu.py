@@ -164,12 +164,13 @@ def test_batched_windows(ctx):
         _same_summary(sums[i], o)
 
 
-@pytest.mark.parametrize("cams_per_window", [(10, 17, 5, 24), (24, 10), (14, 10, 16, 3), (8, 10, 11, 10)])
+@pytest.mark.parametrize("cams_per_window", [(10, 17, 5, 24), (24, 10), (14, 10, 16, 3), (8, 10, 11, 10), (40, 10)])
 def test_batched_windows_of_mixed_solver_paths(ctx, cams_per_window):
     """One batch, windows of different accumulation paths (dense <= 10 cameras, privatised <= 16,
     work lists beyond): the build kernels are chosen per launch, so one window with 6C > 96 moves
     the whole batch onto the work-list path and every window needs its lists (the soak found
-    batches with such a window returning garbage for all their windows)."""
+    batches with such a window returning garbage for all their windows).  A batch with 6C > 143 factorises
+    on the multi-kernel panel / update Cholesky: 5 block columns for 24 cameras, 8 for 40."""
     pbs = [synth.make_ba_problem(300 + 7 * i + C, C=C, P=120 + 30 * i, obs_per_point=(3, 4, min(C, 6)),
                                  traj_len=float(max(3.0, 0.4 * C))) for i, C in enumerate(cams_per_window)]
     bt = synth.batch_windows(pbs)

@@ -32,7 +32,7 @@ def test_golden_cv2(ctx, golden_dir):
 
 @pytest.mark.parametrize("mode", [0, 1])
 @pytest.mark.parametrize("shape", [(1, 1), (1, 77), (77, 1), (31, 33), (128, 256), (129, 257),
-                                   (1000, 1000), (2000, 2000), (300, 5000), (5000, 300)])
+                                   (1000, 1000), (1300, 2100), (2000, 2000), (300, 5000), (5000, 300)])
 def test_crosscheck_vs_oracle(ctx, shape, mode):
     rng = np.random.default_rng(hash(shape) % 2**32 + mode)
     for kind in ("uniform", "tie"):
@@ -75,6 +75,11 @@ def test_knn2_ratio(ctx):
     assert np.array_equal(idx, oi) and np.array_equal(dist, od)
     exp = (od[:, 0] <= 100) & (od[:, 0].astype(np.float32) < np.float32(0.8) * od[:, 1].astype(np.float32))
     assert np.array_equal(ok.astype(bool), exp)
+    # a low-entropy train set: best and second best are decided by the lowest-index rule
+    q, t = synth.descriptors_uniform(1300, rng), synth.descriptors_tie_stress(2100, rng, 2, 3)
+    idx, dist, _ = ctx.match_knn2(q, t)
+    oi, od = ref.knn2(q, t)
+    assert np.array_equal(idx, oi) and np.array_equal(dist, od)
 
 
 def test_properties_full_size(ctx):

@@ -68,6 +68,9 @@ def test_points_edge_cases(ctx):
     pts0 = synth.make_proj_points(synth.make_frame(10, seed=1), 50, seed=2)
     r = ctx.search_proj_points(fr0, pts0, 1.0)
     assert r["n_matches"] == 0
+    # a very large frame: 15 000 keypoints
+    big = synth.make_frame(15000, seed=15000, stereo=True, claimed_frac=0.2)
+    _cmp_points(ctx, big, synth.make_proj_points(big, 3000, seed=15000, nobs=(0, 1, 2), inactive_frac=0.1), 1.0)
 
 
 @pytest.mark.parametrize("motion", ["forward", "backward", "still"])
