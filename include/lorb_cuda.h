@@ -524,6 +524,56 @@ int lorb_ba_pose_only(lorb_ctx* ctx, int n, const float* xw, const float* uv, co
                       double* rt, const lorb_ba_options* opt, lorb_ba_summary* summary);
 
 /*
+ * Pose-only BA with outlier rounds (beyond the reference; ORB-SLAM2's Optimizer::PoseOptimization),
+ * for a batch of frames.  Frame f owns observations [obs_off[f], obs_off[f+1]) of xw / uv / info
+ * and the pose rt[6f .. 6f+6).
+ *   obs_off [n_frames+1] int, obs_off[0] = 0, non-decreasing; O = obs_off[n_frames]
+ *   xw [O x 3], uv [O x 2] float    as lorb_ba_pose_only
+ *   info [O] float or NULL          per-observation weight w (NULL = 1), e.g. 1 / sigma^2 of the octave
+ *   K = {fx, fy, cx, cy} float      shared by every frame
+ *   rt [n_frames x 6] double in/out
+ *   out_inlier [O]                  1 = inlier, 0 = outlier
+ *   out_chi2 [O] or NULL            w |r|^2 of each observation
+ *   n_inliers [n_frames]            number of inliers of each frame
+ *   rounds_run [n_frames] or NULL   rounds each frame ran
+ *   summaries [n_frames x n_rounds] or NULL   LM summary of every round of every frame
+ * Semantics:
+ * - The residual is PoseCost, with its fx-for-v quirk (ba_math.cuh::obs_eval, as lorb_ba_pose_only).
+ * - A weighted observation is the residual sqrt(w) r.  The ctx's robust loss (lorb_ba_set_loss)
+ *   applies to s = w |r|^2, as in Ceres with a scaled cost function and a LossFunction.  With a loss
+ *   set, its scale is therefore in whitened units.
+ * - Each round is one full solve under the Ceres contract of lorb_ba_pose_only, with opt as its budget:
+ *   - it starts from the input pose, as ORB-SLAM2 resets to pFrame->mTcw every round;
+ *   - it has a fresh trust region and Jacobi scaling;
+ *   - it runs over the observations flagged inlier at its start.  Round 0 starts with all of them.
+ * - After a round, every observation of the frame is classified at that round's pose: inlier iff
+ *   w |r|^2 <= chi2.  This chi^2 is the unrobustified one.
+ * - If fewer than 3 observations are inliers at the start of a round, that round and the rest are
+ *   skipped.
+ * - rt, out_inlier, out_chi2 and n_inliers always describe the returned pose.  That is the pose after
+ *   the last round that ran, or the input pose with its classification if no round ran.
+ * - Summary slots of rounds that did not run are zero-filled.
+ * - Refused with LORB_ERR_ARG, before any device work: bad offsets, a weight that is not finite and
+ *   > 0, or an out-of-range rounds field.
+ * - n_frames = 0 is a no-op.
+ * One CTA per frame, all rounds of all frames in one launch; a frame's result is bit-identical whether
+ * it is solved alone or in a batch.
+ */
+typedef struct lorb_ba_pose_rounds {
+  int n_rounds;       /* 4     (1..16) */
+  int robust_rounds;  /* 3     rounds [0, robust_rounds) use the ctx's loss, later rounds plain least squares (0..n_rounds) */
+  double chi2;        /* 5.991 chi-square threshold on w*|r|^2 (finite, > 0) */
+} lorb_ba_pose_rounds;
+void lorb_ba_default_pose_rounds(lorb_ba_pose_rounds* r);
+
+int lorb_ba_pose_rounds_batched(lorb_ctx* ctx, int n_frames, const int* obs_off /* [n_frames+1] */,
+    const float* xw /* [O x 3] */, const float* uv /* [O x 2] */, const float* info /* [O] or NULL = 1 */,
+    const float* K /* fx fy cx cy, shared */, double* rt /* [n_frames x 6] in/out */,
+    const lorb_ba_pose_rounds* rounds, const lorb_ba_options* opt /* per round */,
+    uint8_t* out_inlier /* [O] */, double* out_chi2 /* [O] or NULL */, int* n_inliers /* [n_frames] */,
+    int* rounds_run /* [n_frames] or NULL */, lorb_ba_summary* summaries /* [n_frames x n_rounds] or NULL */);
+
+/*
  * BA::LocalPoseOptimization (reference src/bundle_adjust.cpp:207-330).
  *   cams [C x 6] double in/out   (w0,w1,w2,t0,t1,t2) per window frame (:250-255)
  *   pts  [P x 3] double in/out   (:262-264)

@@ -35,6 +35,7 @@ EXPORTS = [
     "lorb_ba_default_options", "lorb_ba_pose_only", "lorb_ba_local", "lorb_ba_local_batched", "lorb_ba_local_shard",
     "lorb_ba_problem_create", "lorb_ba_problem_create_batched", "lorb_ba_problem_create_sharded", "lorb_shard_range", "lorb_ba_shard_points", "lorb_set_host_threads", "lorb_ba_problem_reset", "lorb_ba_problem_solve",
     "lorb_ba_problem_download", "lorb_ba_problem_destroy", "lorb_ba_set_loss", "lorb_ba_get_loss",
+    "lorb_ba_default_pose_rounds", "lorb_ba_pose_rounds_batched",
     "lorb_dist_get_unique_id",
     "lorb_dist_init", "lorb_dist_finalize", "lorb_dist_allreduce_f64", "lorb_microbench_popc",
     "lorb_microbench_fp64", "lorb_microbench_tensor_i8", "lorb_ctx_profile", "lorb_ctx_profile_read",
@@ -67,6 +68,10 @@ class BASummary(C.Structure):
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+class PoseRounds(C.Structure):
+    _fields_ = [("n_rounds", C.c_int), ("robust_rounds", C.c_int), ("chi2", C.c_double)]
 
 
 class FrameView(C.Structure):
@@ -151,6 +156,17 @@ def ba_options(**kw):
             raise AttributeError(k)
         setattr(o, k, v)
     return o
+
+
+def pose_rounds_options(**kw):
+    """lorb_ba_pose_rounds with ORB-SLAM2's defaults (4 rounds, 3 robust, chi2 5.991), fields overridden by kw."""
+    r = PoseRounds()
+    load_library().lorb_ba_default_pose_rounds(C.byref(r))
+    for k, v in kw.items():
+        if not hasattr(r, k):
+            raise AttributeError(k)
+        setattr(r, k, v)
+    return r
 
 
 def _frame_view(fr):
@@ -537,6 +553,36 @@ class Context:
         _check(self._lib.lorb_ba_pose_only(self._h, len(xw), _ptr(xw), _ptr(uv), _ptr(K), _ptr(rt),
                                            C.byref(opt), C.byref(s)))
         return rt, s.as_dict()
+
+    def ba_pose_rounds(self, xw, uv, K, rt, info=None, rounds=None, opt=None):
+        """One frame of ba_pose_rounds_batched -> (rt, inlier[n] bool, chi2[n], n_inliers, rounds_run,
+        summaries[n_rounds])."""
+        n = len(_arr(xw, np.float32).reshape(-1, 3))
+        rt, inl, chi2, n_in, run, sums = self.ba_pose_rounds_batched(
+            [0, n], xw, uv, K, _arr(rt, np.float64).reshape(1, 6), info, rounds, opt)
+        return rt[0], inl, chi2, int(n_in[0]), int(run[0]), sums[0]
+
+    def ba_pose_rounds_batched(self, obs_off, xw, uv, K, rt, info=None, rounds=None, opt=None):
+        """lorb_ba_pose_rounds_batched: frame f owns observations obs_off[f]:obs_off[f+1] and pose rt[f].
+        -> (rt[F,6], inlier[O] bool, chi2[O], n_inliers[F], rounds_run[F], summaries: F lists of n_rounds
+        dicts)."""
+        oo = _arr(obs_off, np.int32).reshape(-1)
+        xw, uv = _arr(xw, np.float32).reshape(-1, 3), _arr(uv, np.float32).reshape(-1, 2)
+        K = _arr(K, np.float32).reshape(4)
+        rt = _arr(rt, np.float64).reshape(-1, 6).copy()
+        w = None if info is None else _arr(info, np.float32).reshape(-1)
+        rounds = rounds or pose_rounds_options()
+        opt = opt or ba_options()
+        F, O = len(rt), len(xw)
+        inl, chi2 = np.zeros(O, np.uint8), np.zeros(O, np.float64)
+        n_in, run = np.zeros(F, np.int32), np.zeros(F, np.int32)
+        sums = (BASummary * max(1, F * rounds.n_rounds))()
+        _check(self._lib.lorb_ba_pose_rounds_batched(
+            self._h, F, _ptr(oo), _ptr(xw), _ptr(uv), _ptr(w), _ptr(K), _ptr(rt), C.byref(rounds),
+            C.byref(opt), _ptr(inl), _ptr(chi2), _ptr(n_in), _ptr(run), sums))
+        R = rounds.n_rounds
+        return (rt, inl.astype(bool), chi2, n_in, run,
+                [[sums[f * R + r].as_dict() for r in range(R)] for f in range(F)])
 
     def ba_local_shard(self, pb, opt=None):
         """lorb_ba_local_shard: `pb` is this rank's shard; collective over the ctx communicator."""

@@ -12,6 +12,7 @@
 #include "../include/bundle_adjust.h"
 #include "../include/matcher.h"
 #include "../include/local_map_index.h"
+#include "../include/pose_optimization.h"
 
 #include <algorithm>
 #include <chrono>
@@ -171,6 +172,59 @@ int harness_proj_frame(int n_kp, const float* x, const float* y, const int* oct,
 		else out_state[i] = -1;
 	}
 	return (int)n;
+}
+
+// The tracking loop with outlier rounds: lorb_host::PoseOptimization on Last (keypoints luv, octaves
+// loct, valid map points xw; rt float[6] R then T in/out), then Matcher::SearchByProjection(Cur, Last, th)
+// on the same Last object, which reads the mvbOutlier flags PoseOptimization set.  Out: Last's
+// mvbOutlier (1 = outlier, 0 otherwise), its mTcw after SetPose, Cur's state as harness_proj_frame,
+// the number of matches in *n_matches.  Returns PoseOptimization's inlier count.
+int harness_pose_rounds_search(int n_kp, const float* x, const float* y, const int* oct, const float* ang,
+                               const float* ur, const uint8_t* desc, float minx, float maxx, float miny,
+                               float maxy, int nlev, const float* sf, const float* tcw_cur, const float* K6,
+                               int n_last, const uint8_t* valid, const float* xw, const int* loct,
+                               const float* lang, const float* luv, const uint8_t* mpdesc, const int* nobs,
+                               float* rt, float th, uint8_t* out_outlier, float* out_tcw_last, int* out_state,
+                               int* n_matches)
+{
+	Camera cam;
+	cam.fx = K6[0]; cam.fy = K6[1]; cam.cx = K6[2]; cam.cy = K6[3];
+	Frame Cur, Last;
+	std::vector<float> lz(n_last, 0.0f), lur(n_last, -1.0f);
+	std::vector<uint8_t> ldesc((size_t)n_last*32, 0);
+	FillFrame(Last, n_last, lz.data(), lz.data(), loct, lang, lur.data(), ldesc.data(), minx, maxx, miny, maxy,
+	          nlev, sf);
+	Last.mpCamera = &cam;
+	std::vector<MapPoint> mps(n_last);
+	for(int i=0;i<n_last;i++)
+	{
+		Last.mvKeysUn[i].pt = cv::Point2f(luv[2*i], luv[2*i+1]);
+		if(valid[i])
+		{
+			mps[i].mWorldPos = cv::Point3f(xw[3*i], xw[3*i+1], xw[3*i+2]);
+			mps[i].mDescriptor = DescMat(mpdesc + (size_t)i*32, 1);
+			mps[i].mnObs = (size_t)nobs[i];
+			Last.mvpMapPoints[i] = &mps[i];
+		}
+	}
+	for(int k=0;k<3;k++) { Last.mRvec.at<float>(k) = rt[k]; Last.mTvec.at<float>(k) = rt[3+k]; }
+	const int n_in = lorb_host::PoseOptimization(&Last);
+	for(int k=0;k<3;k++) { rt[k] = Last.mRvec.at<float>(k); rt[3+k] = Last.mTvec.at<float>(k); }
+	for(int i=0;i<n_last;i++) out_outlier[i] = Last.mvbOutlier[i] ? 1 : 0;
+	for(int r=0;r<4;r++) for(int c=0;c<4;c++) out_tcw_last[4*r+c] = Last.mTcw.at<float>(r,c);
+
+	FillFrame(Cur, n_kp, x, y, oct, ang, ur, desc, minx, maxx, miny, maxy, nlev, sf);
+	Cur.fx = K6[0]; Cur.fy = K6[1]; Cur.cx = K6[2]; Cur.cy = K6[3]; Cur.mbf = K6[4]; Cur.mb = K6[5];
+	for(int r=0;r<4;r++) for(int c=0;c<4;c++) Cur.mTcw.at<float>(r,c) = tcw_cur[4*r+c];
+	*n_matches = (int)Matcher::SearchByProjection(&Cur, &Last, th);
+	for(int i=0;i<n_kp;i++)
+	{
+		MapPoint* h = Cur.mvpMapPoints[i];
+		if(h == NULL) out_state[i] = -2;
+		else if(n_last && h >= &mps[0] && h <= &mps[n_last-1]) out_state[i] = (int)(h - &mps[0]);
+		else out_state[i] = -1;
+	}
+	return n_in;
 }
 
 // BA::ProjectPoseOptimization: rt (float[6]: R then T) in/out
