@@ -618,6 +618,74 @@ int lorb_ba_local_batched(lorb_ctx* ctx, int n_windows, const int* cam_off, doub
                           const int* fix_pt, const float* fix_uv, const float* fix_rt,
                           const float* K, const lorb_ba_options* opt, lorb_ba_summary* summaries);
 
+/*
+ * Local BA with outlier rounds (beyond the reference; ORB-SLAM2's Optimizer::LocalBundleAdjustment),
+ * for a batch of windows in the layout of lorb_ba_local_batched.
+ *   obs_w [O] float or NULL         per-observation weight w of the in-window observations (NULL = 1),
+ *                                   e.g. 1 / sigma^2 of the keypoint's octave; indexed like obs_cam
+ *   fix_w [F] float or NULL         the same for the fixed observations; indexed like fix_pt
+ *   rounds, opt [n_rounds]          round r runs under opt[r]
+ *   obs_inlier [O], fix_inlier [F]  1 = inlier, 0 = outlier
+ *   obs_chi2 [O], fix_chi2 [F]      w |r|^2 of each observation (either may be NULL)
+ *   n_inliers [n_windows]           in-window + fixed inliers of each window
+ *   summaries [n_windows x n_rounds] or NULL   LM summary of every round of every window
+ * Semantics:
+ * - Residuals: PoseMPCost for in-window observations, MPCost with the float pose for fixed observers,
+ *   as lorb_ba_local.
+ * - A weighted observation is the residual sqrt(w) r.  The ctx's robust loss (lorb_ba_set_loss)
+ *   applies to s = w |r|^2, so its scale is in whitened units.
+ * - Each round is one full LM solve under opt[r], with a fresh trust region and Jacobi scaling taken
+ *   at the round's start from the weighted Jacobian of its inliers:
+ *   - it runs over the observations flagged inlier at its start.  Round 0 runs over all of them;
+ *   - rounds [0, robust_rounds) use the ctx's loss, later rounds plain least squares;
+ *   - it starts from the previous round's result, not from the input, as ORB-SLAM2's
+ *     LocalBundleAdjustment continues where its first optimisation stopped.
+ * - A camera or point with no inlier observation keeps its value bit for bit through the round.  It
+ *   stays in |x| of the parameter-tolerance test (Ceres would drop such a block from its program;
+ *   only that test differs).
+ * - After each round, every observation of the window (in-window and fixed, inlier or not) is
+ *   classified at that round's parameters: inlier iff w |r|^2 <= chi2 and, with depth_check, the
+ *   point's depth in the observing camera is > 0.  This chi^2 is the unrobustified one.
+ * - A window with no inliers still runs its round: it stops at its first gradient test
+ *   (LORB_BA_CONV_GRADIENT, 0 iterations).
+ * - cams, pts, the flags, chi^2 values and counts describe the returned parameters, i.e. the
+ *   classification after the last round.  Flags and chi^2 are in the caller's order.
+ * - Every window runs its own LM loop in every round; the rounds run in lockstep across the batch.
+ * - Refused with LORB_ERR_ARG, before any device work and with the outputs untouched: whatever
+ *   lorb_ba_local_batched refuses, a weight that is not finite and > 0, an out-of-range rounds field,
+ *   opt NULL, or a NULL inlier array for a side (in-window / fixed) with observations.
+ * - n_windows = 0 is a no-op.
+ * Not sharded: the rounds run on one GPU.
+ */
+typedef struct lorb_ba_local_rounds {
+  int n_rounds;       /* 2     (1..16) */
+  int robust_rounds;  /* 1     rounds [0, robust_rounds) use the ctx's loss, later rounds plain least squares (0..n_rounds) */
+  double chi2;        /* 5.991 threshold on w*|r|^2 (finite, > 0) */
+  int depth_check;    /* 1     0/1: an observation whose point is not in front of its camera (z <= 0) is an outlier */
+  int reserved;
+} lorb_ba_local_rounds;
+/* ORB-SLAM2's LocalBundleAdjustment settings; opt2 (may be NULL) receives two lorb_ba_default_options
+ * with max_num_iterations 5 and 10. */
+void lorb_ba_default_local_rounds(lorb_ba_local_rounds* r, lorb_ba_options* opt2);
+
+int lorb_ba_local_rounds_batched(lorb_ctx* ctx, int n_windows, const int* cam_off, double* cams,
+    const int* pt_off, double* pts, const int* obs_off, const int* obs_cam, const int* obs_pt,
+    const float* obs_uv, const float* obs_w /* [O] or NULL = 1 */,
+    const int* fix_off /* or NULL */, const int* fix_pt, const float* fix_uv, const float* fix_rt,
+    const float* fix_w /* [F] or NULL = 1 */, const float* K,
+    const lorb_ba_local_rounds* rounds, const lorb_ba_options* opt /* [n_rounds], round r runs under opt[r] */,
+    uint8_t* obs_inlier /* [O] */, double* obs_chi2 /* [O] or NULL */,
+    uint8_t* fix_inlier /* [F] */, double* fix_chi2 /* [F] or NULL */,
+    int* n_inliers /* [n_windows], in-window + fixed */, lorb_ba_summary* summaries /* [n_windows x n_rounds] or NULL */);
+/* The same for one window, in the argument layout of lorb_ba_local (the name lorb_ba_local_rounds is
+ * the settings type). */
+int lorb_ba_local_rounds_single(lorb_ctx* ctx, int C, double* cams, int P, double* pts, int O,
+    const int* obs_cam, const int* obs_pt, const float* obs_uv, const float* obs_w, int F,
+    const int* fix_pt, const float* fix_uv, const float* fix_rt, const float* fix_w, const float* K,
+    const lorb_ba_local_rounds* rounds, const lorb_ba_options* opt,
+    uint8_t* obs_inlier, double* obs_chi2, uint8_t* fix_inlier, double* fix_chi2,
+    int* n_inliers /* [1] */, lorb_ba_summary* summaries /* [n_rounds] or NULL */);
+
 /* Team size of the library's host-side staging loops (OpenMP) for the calling thread.  Launchers
  * such as torchrun export OMP_NUM_THREADS=1 to every rank; a host that knows how many ranks share
  * the box hands each its share of the cores here.  (omp_set_num_threads on the process's OpenMP

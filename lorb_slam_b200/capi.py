@@ -36,6 +36,7 @@ EXPORTS = [
     "lorb_ba_problem_create", "lorb_ba_problem_create_batched", "lorb_ba_problem_create_sharded", "lorb_shard_range", "lorb_ba_shard_points", "lorb_set_host_threads", "lorb_ba_problem_reset", "lorb_ba_problem_solve",
     "lorb_ba_problem_download", "lorb_ba_problem_destroy", "lorb_ba_set_loss", "lorb_ba_get_loss",
     "lorb_ba_default_pose_rounds", "lorb_ba_pose_rounds_batched",
+    "lorb_ba_default_local_rounds", "lorb_ba_local_rounds_batched", "lorb_ba_local_rounds_single",
     "lorb_dist_get_unique_id",
     "lorb_dist_init", "lorb_dist_finalize", "lorb_dist_allreduce_f64", "lorb_microbench_popc",
     "lorb_microbench_fp64", "lorb_microbench_tensor_i8", "lorb_ctx_profile", "lorb_ctx_profile_read",
@@ -72,6 +73,11 @@ class BASummary(C.Structure):
 
 class PoseRounds(C.Structure):
     _fields_ = [("n_rounds", C.c_int), ("robust_rounds", C.c_int), ("chi2", C.c_double)]
+
+
+class LocalRounds(C.Structure):
+    _fields_ = [("n_rounds", C.c_int), ("robust_rounds", C.c_int), ("chi2", C.c_double), ("depth_check", C.c_int),
+                ("reserved", C.c_int)]
 
 
 class FrameView(C.Structure):
@@ -167,6 +173,39 @@ def pose_rounds_options(**kw):
             raise AttributeError(k)
         setattr(r, k, v)
     return r
+
+
+def local_rounds_options(**kw):
+    """lorb_ba_local_rounds with ORB-SLAM2's LocalBundleAdjustment defaults (2 rounds, 1 robust, chi2 5.991,
+    depth check), fields overridden by kw."""
+    r = LocalRounds()
+    load_library().lorb_ba_default_local_rounds(C.byref(r), None)
+    for k, v in kw.items():
+        if not hasattr(r, k):
+            raise AttributeError(k)
+        setattr(r, k, v)
+    return r
+
+
+def local_rounds_budgets():
+    """The two lorb_ba_options of lorb_ba_default_local_rounds: 5 and 10 iterations."""
+    o = (BAOptions * 2)()
+    load_library().lorb_ba_default_local_rounds(None, o)
+    return [o[0], o[1]]
+
+
+def _round_opts(rounds, opt):
+    """opt: None (the default budgets when there are two rounds, else default options), one BAOptions for
+    every round, or a list of n_rounds of them -> a ctypes array."""
+    R = rounds.n_rounds
+    if opt is None:
+        opt = local_rounds_budgets() if R == 2 else [ba_options() for _ in range(R)]
+    elif isinstance(opt, BAOptions):
+        opt = [opt] * R
+    arr = (BAOptions * max(1, len(opt)))()
+    for i, o in enumerate(opt):
+        arr[i] = o
+    return arr
 
 
 def _frame_view(fr):
@@ -583,6 +622,67 @@ class Context:
         R = rounds.n_rounds
         return (rt, inl.astype(bool), chi2, n_in, run,
                 [[sums[f * R + r].as_dict() for r in range(R)] for f in range(F)])
+
+    def ba_local_rounds(self, pb, w=None, fix_w=None, rounds=None, opt=None):
+        """lorb_ba_local_rounds_single on one window (the dict of ba_local); w [O] / fix_w [F] weights or None.
+        -> (cams, pts, obs_inlier[O] bool, obs_chi2[O], fix_inlier[F] bool, fix_chi2[F], n_inliers,
+        summaries[n_rounds])."""
+        cams = _arr(pb["cams"], np.float64).copy()
+        pts = _arr(pb["pts"], np.float64).copy()
+        oc, op = _arr(pb["obs_cam"], np.int32), _arr(pb["obs_pt"], np.int32)
+        ouv = _arr(pb["obs_uv"], np.float32)
+        fp = _arr(pb.get("fix_pt", np.zeros(0)), np.int32)
+        fuv = _arr(pb.get("fix_uv", np.zeros((0, 2))), np.float32)
+        frt = _arr(pb.get("fix_rt", np.zeros((0, 6))), np.float32)
+        K = _arr(pb["K"], np.float32).reshape(4)
+        w = None if w is None else _arr(w, np.float32).reshape(-1)
+        fw = None if fix_w is None else _arr(fix_w, np.float32).reshape(-1)
+        rounds = rounds or local_rounds_options()
+        opts = _round_opts(rounds, opt)
+        O, F, R = len(oc), len(fp), rounds.n_rounds
+        inl, chi2 = np.zeros(O, np.uint8), np.zeros(O, np.float64)
+        finl, fchi2 = np.zeros(F, np.uint8), np.zeros(F, np.float64)
+        n_in = np.zeros(1, np.int32)
+        sums = (BASummary * R)()
+        _check(self._lib.lorb_ba_local_rounds_single(
+            self._h, len(cams), _ptr(cams), len(pts), _ptr(pts), O, _ptr(oc), _ptr(op), _ptr(ouv), _ptr(w), F,
+            _ptr(fp), _ptr(fuv), _ptr(frt), _ptr(fw), _ptr(K), C.byref(rounds), opts, _ptr(inl), _ptr(chi2),
+            _ptr(finl), _ptr(fchi2), _ptr(n_in), sums))
+        return (cams, pts, inl.astype(bool), chi2, finl.astype(bool), fchi2, int(n_in[0]),
+                [s.as_dict() for s in sums])
+
+    def ba_local_rounds_batched(self, bt, w=None, fix_w=None, rounds=None, opt=None):
+        """lorb_ba_local_rounds_batched on the windows of synth.batch_windows (the dict of ba_local_batched).
+        -> (cams, pts, obs_inlier[O] bool, obs_chi2[O], fix_inlier[F] bool, fix_chi2[F], n_inliers[n_windows],
+        summaries: n_windows lists of n_rounds dicts)."""
+        cams = _arr(bt["cams"], np.float64).copy()
+        pts = _arr(bt["pts"], np.float64).copy()
+        co, po, oo = (_arr(bt[k], np.int32) for k in ("cam_off", "pt_off", "obs_off"))
+        oc, op = _arr(bt["obs_cam"], np.int32), _arr(bt["obs_pt"], np.int32)
+        ouv = _arr(bt["obs_uv"], np.float32)
+        K = _arr(bt["K"], np.float32).reshape(4)
+        nw = int(bt["n_windows"])
+        fo = fp = fuv = frt = None
+        F = 0
+        if "fix_off" in bt:
+            fo, fp = _arr(bt["fix_off"], np.int32), _arr(bt["fix_pt"], np.int32)
+            fuv, frt = _arr(bt["fix_uv"], np.float32), _arr(bt["fix_rt"], np.float32)
+            F = len(fp)
+        w = None if w is None else _arr(w, np.float32).reshape(-1)
+        fw = None if fix_w is None else _arr(fix_w, np.float32).reshape(-1)
+        rounds = rounds or local_rounds_options()
+        opts = _round_opts(rounds, opt)
+        O, R = len(oc), rounds.n_rounds
+        inl, chi2 = np.zeros(O, np.uint8), np.zeros(O, np.float64)
+        finl, fchi2 = np.zeros(F, np.uint8), np.zeros(F, np.float64)
+        n_in = np.zeros(max(nw, 1), np.int32)
+        sums = (BASummary * max(1, nw * R))()
+        _check(self._lib.lorb_ba_local_rounds_batched(
+            self._h, nw, _ptr(co), _ptr(cams), _ptr(po), _ptr(pts), _ptr(oo), _ptr(oc), _ptr(op), _ptr(ouv), _ptr(w),
+            _ptr(fo), _ptr(fp), _ptr(fuv), _ptr(frt), _ptr(fw), _ptr(K), C.byref(rounds), opts, _ptr(inl),
+            _ptr(chi2), _ptr(finl), _ptr(fchi2), _ptr(n_in), sums))
+        return (cams, pts, inl.astype(bool), chi2, finl.astype(bool), fchi2, n_in[:nw],
+                [[sums[i * R + r].as_dict() for r in range(R)] for i in range(nw)])
 
     def ba_local_shard(self, pb, opt=None):
         """lorb_ba_local_shard: `pb` is this rank's shard; collective over the ctx communicator."""

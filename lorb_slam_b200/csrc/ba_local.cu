@@ -24,6 +24,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <new>
 #include <vector>
 
@@ -75,6 +76,55 @@ struct BADev {
   double loss_scale;
 };
 
+// Descriptor of an outlier-round solve (lorb_ba_local_rounds_batched), read by the WEIGHTED kernel
+// instantiations and the round kernels only.  It extends BADev instead of adding to it, so that BADev,
+// and with it the code of every existing instantiation, stays as it was.  Arrays in CSR order.
+struct BADevW : BADev {
+  double* obs_sw;        // sqrt of the effective weight: sqrt(w) for an inlier, 0 for an outlier
+  const float* obs_w;    // the caller's weight w (the chi-square test)
+  uint8_t* obs_in;       // inlier flag of the last classification
+  double* obs_chi2;      // w |r|^2 of the last classification
+  int* n_in;             // inliers of the window
+};
+
+template <bool WEIGHTED>
+struct DescOf {
+  using T = BADev;
+};
+template <>
+struct DescOf<true> {
+  using T = BADevW;
+};
+
+// The descriptor of window `w`: a WEIGHTED launch passes its BADevW array through the BADev pointer.
+template <bool WEIGHTED>
+__device__ __forceinline__ typename DescOf<WEIGHTED>::T load_desc(const BADev* __restrict__ probs, int w) {
+  return reinterpret_cast<const typename DescOf<WEIGHTED>::T*>(probs)[w];
+}
+
+// A weighted observation is the residual sqrt(w) r: r and its Jacobian blocks (Jc may be null) are
+// scaled ahead of the loss.  An outlier (effective weight 0) leaves r = 0, J = 0 and rho = 0 exactly,
+// by selection, so that a non-finite residual of an outlier (a point crossing its camera's plane in a
+// trial step) cannot turn into 0 * inf = NaN.
+__device__ __forceinline__ void apply_weight(const BADev&, int, double*, double*, double*) {}
+__device__ __forceinline__ void apply_weight(const BADevW& p, int o, double r[2], double* Jc, double* Jp) {
+  const double sw = p.obs_sw[o];
+  const bool in = sw != 0.0;
+  r[0] = in ? r[0] * sw : 0.0;
+  r[1] = in ? r[1] * sw : 0.0;
+  if (Jc) {
+#pragma unroll
+    for (int k = 0; k < 12; k++) Jc[k] = in ? Jc[k] * sw : 0.0;
+  }
+#pragma unroll
+  for (int k = 0; k < 6; k++) Jp[k] = in ? Jp[k] * sw : 0.0;
+}
+__device__ __forceinline__ double weigh_sq(const BADev&, int, double s) { return s; }
+__device__ __forceinline__ double weigh_sq(const BADevW& p, int o, double s) {
+  const double sw = p.obs_sw[o];
+  return sw != 0.0 ? sw * sw * s : 0.0;
+}
+
 __device__ __forceinline__ int upper_idx(int a, int b) {  // a <= b, 6x6
   return a * 6 - (a * (a - 1)) / 2 + (b - a);
 }
@@ -110,13 +160,14 @@ __global__ void ba_camrot_kernel(const BADev* __restrict__ probs, int which /*0 
   cam_rotation(p.cams[buf] + 6 * c, p.camrot[buf] + CAMROT * c, true);
 }
 
-// Observation of point X by window camera `cam` (>= 0) at pixel uv, with scaled Jacobians.
+// Observation `o` of point X by window camera `cam` (>= 0) at pixel uv, with scaled Jacobians.
 // ROBUST: r and the Jacobians come out corrected by the solve's loss (robust_correct) and *rho, when
 // given, receives rho(|r|^2); the kernels are instantiated with ROBUST = false for plain least
-// squares, which keeps that path exactly the code it was.
-template <bool ROBUST = false>
-__device__ __forceinline__ void eval_obs_cam(const BADev& p, const double* __restrict__ cams,
-                                             const double* __restrict__ camrot, int cam, float2 uv,
+// squares, which keeps that path exactly the code it was.  With a BADevW descriptor (the WEIGHTED
+// instantiations, always ROBUST) the observation's weight is applied ahead of the loss.
+template <bool ROBUST = false, typename D = BADev>
+__device__ __forceinline__ void eval_obs_cam(const D& p, const double* __restrict__ cams,
+                                             const double* __restrict__ camrot, int cam, int o, float2 uv,
                                              const double X[3], const double sp[3], double r[2], double Jc[12],
                                              double Jp[6], double* rho = nullptr) {
   const double* t = cams + 6 * cam + 3;
@@ -134,21 +185,22 @@ __device__ __forceinline__ void eval_obs_cam(const BADev& p, const double* __res
     Jp[3 + a] *= sp[a];
   }
   if (ROBUST) {
+    apply_weight(p, o, r, Jc, Jp);
     const double q = robust_correct(p.loss_kind, p.loss_scale, r, Jc, Jp);
     if (rho) *rho = q;
   }
 }
 
 // Evaluate observation `o` of point X with scaled Jacobians (ROBUST, rho: as eval_obs_cam).
-template <bool ROBUST = false>
-__device__ __forceinline__ int eval_obs(const BADev& p, const double* __restrict__ cams,
+template <bool ROBUST = false, typename D = BADev>
+__device__ __forceinline__ int eval_obs(const D& p, const double* __restrict__ cams,
                                         const double* __restrict__ camrot, int o, const double X[3],
                                         const double sp[3], double r[2], double Jc[12],
                                         double Jp[6], double* rho = nullptr) {
   const int cam = p.obs_cam[o];
   const float2 uv = p.obs_uv[o];
   if (cam >= 0) {
-    eval_obs_cam<ROBUST>(p, cams, camrot, cam, uv, X, sp, r, Jc, Jp, rho);
+    eval_obs_cam<ROBUST>(p, cams, camrot, cam, o, uv, X, sp, r, Jc, Jp, rho);
     return cam;
   }
   const double* f = p.fixrt + 12 * (size_t)(-1 - cam);
@@ -160,6 +212,7 @@ __device__ __forceinline__ int eval_obs(const BADev& p, const double* __restrict
     Jp[3 + a] *= sp[a];
   }
   if (ROBUST) {
+    apply_weight(p, o, r, nullptr, Jp);
     const double q = robust_correct(p.loss_kind, p.loss_scale, r, nullptr, Jp);
     if (rho) *rho = q;
   }
@@ -187,8 +240,8 @@ __device__ __forceinline__ void cs_fill(const BADev& p, const double* __restrict
 }
 
 // eval_obs with the window's cameras in shared memory (same arithmetic, same order).
-template <bool ROBUST = false>
-__device__ __forceinline__ int eval_obs_cs(const BADev& p, const double* __restrict__ cs, int stride, int o,
+template <bool ROBUST = false, typename D = BADev>
+__device__ __forceinline__ int eval_obs_cs(const D& p, const double* __restrict__ cs, int stride, int o,
                                            const double X[3], const double sp[3], double r[2], double Jc[12],
                                            double Jp[6], double* rho = nullptr) {
   const int cam = p.obs_cam[o];
@@ -213,18 +266,20 @@ __device__ __forceinline__ int eval_obs_cs(const BADev& p, const double* __restr
     Jp[3 + a] *= sp[a];
   }
   if (ROBUST) {
+    apply_weight(p, o, r, cam >= 0 ? Jc : nullptr, Jp);
     const double q = robust_correct(p.loss_kind, p.loss_scale, r, cam >= 0 ? Jc : nullptr, Jp);
     if (rho) *rho = q;
   }
   return cam;
 }
 
-// Candidate cost of one observation with squared residual norm s: rho(s) under the solve's loss.
-template <bool ROBUST>
-__device__ __forceinline__ double obs_rho(const BADev& p, double s) {
+// Candidate cost of observation `o` with squared residual norm s: rho(w s) under the solve's loss
+// (w = 1 without a BADevW descriptor).
+template <bool ROBUST, typename D>
+__device__ __forceinline__ double obs_rho(const D& p, int o, double s) {
   if (!ROBUST) return s;
   double rho, rho1;
-  loss_eval(p.loss_kind, p.loss_scale, s, rho, rho1);
+  loss_eval(p.loss_kind, p.loss_scale, weigh_sq(p, o, s), rho, rho1);
   return rho;
 }
 
@@ -304,10 +359,10 @@ __device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double
                : "d"(a), "d"(b));
 }
 
-template <bool FULL, int ACC, bool ROBUST = false>
+template <bool FULL, int ACC, bool ROBUST = false, bool WEIGHTED = false>
 __global__ void __launch_bounds__(BA_THREADS)
     ba_build_kernel(const BADev* __restrict__ probs, lorb_ba_options opt, int force) {
-  const BADev p = probs[blockIdx.y];
+  const auto p = load_desc<WEIGHTED>(probs, blockIdx.y);
   LMState* st = p.st;
   if (st->done && !force) return;
   __shared__ int Csm[BA_THREADS];
@@ -623,10 +678,10 @@ __device__ __forceinline__ void dense_reduce(double* __restrict__ Sbuf, double* 
   }
 }
 
-template <bool FULL, bool ROBUST = false>
+template <bool FULL, bool ROBUST = false, bool WEIGHTED = false>
 __global__ void __launch_bounds__(DP_THREADS)
     ba_build_dense_kernel(const BADev* __restrict__ probs, lorb_ba_options opt, int force) {
-  const BADev p = probs[blockIdx.y];
+  const auto p = load_desc<WEIGHTED>(probs, blockIdx.y);
   LMState* st = p.st;
   if (st->done && !force) return;
   __shared__ double red[DP_THREADS / 32];
@@ -871,10 +926,10 @@ __global__ void __launch_bounds__(DP_THREADS)
 // list): one warp accumulates H_cc (21), g_c (6) and the Schur right-hand side
 // W H_pp^-1 g_p (6) of its slice in registers, reduces by shuffles and issues 33
 // atomics per item.
-template <bool ROBUST = false>
+template <bool ROBUST = false, bool WEIGHTED = false>
 __global__ void __launch_bounds__(256)
     ba_cam_rows_kernel(const BADev* __restrict__ probs, int full, int force) {
-  const BADev p = probs[blockIdx.y];
+  const auto p = load_desc<WEIGHTED>(probs, blockIdx.y);
   LMState* st = p.st;
   if (st->done && !force) return;
   const int lane = threadIdx.x & 31;
@@ -900,7 +955,7 @@ __global__ void __launch_bounds__(256)
       X[a] = pts[3 * (size_t)pt + a];
       sp[a] = p.scale_p[3 * (size_t)pt + a];
     }
-    eval_obs_cam<ROBUST>(p, cams, camrot, it.x, uv, X, sp, r, Jc, Jp);
+    eval_obs_cam<ROBUST>(p, cams, camrot, it.x, o, uv, X, sp, r, Jc, Jp);
     int k = 0;
 #pragma unroll
     for (int a = 0; a < 6; a++) {
@@ -945,10 +1000,10 @@ __global__ void __launch_bounds__(256)
 // of one point with camera(i) = ci, camera(j) = cj.  One warp accumulates
 // sum Y_i W_j^T (6x6) in registers over its slice, reduces by shuffles and
 // subtracts it from S with 36 atomics per item (an item is <= 2048 records).
-template <bool ROBUST = false>
+template <bool ROBUST = false, bool WEIGHTED = false>
 __global__ void __launch_bounds__(256)
     ba_schur_pairs_kernel(const BADev* __restrict__ probs) {
-  const BADev p = probs[blockIdx.y];
+  const auto p = load_desc<WEIGHTED>(probs, blockIdx.y);
   LMState* st = p.st;
   if (st->done) return;
   const int lane = threadIdx.x & 31;
@@ -977,7 +1032,7 @@ __global__ void __launch_bounds__(256)
     }
     const double* hi = p.pt_hinv + 6 * (size_t)pt;
     const double h0 = hi[0], h1 = hi[1], h2 = hi[2], h3 = hi[3], h4 = hi[4], h5 = hi[5];
-    eval_obs_cam<ROBUST>(p, cams, camrot, it.x, uvi, X, sp, r, Jc, Jp);
+    eval_obs_cam<ROBUST>(p, cams, camrot, it.x, oi, uvi, X, sp, r, Jc, Jp);
 #pragma unroll
     for (int a = 0; a < 6; a++) {
       const double w0 = Jc[a] * Jp[0] + Jc[6 + a] * Jp[3];
@@ -987,7 +1042,7 @@ __global__ void __launch_bounds__(256)
       Y[3 * a + 1] = w0 * h1 + w1 * h3 + w2 * h4;
       Y[3 * a + 2] = w0 * h2 + w1 * h4 + w2 * h5;
     }
-    if (oj != oi) eval_obs_cam<ROBUST>(p, cams, camrot, it.y, uvj, X, sp, r, Jc, Jp);
+    if (oj != oi) eval_obs_cam<ROBUST>(p, cams, camrot, it.y, oj, uvj, X, sp, r, Jc, Jp);
 #pragma unroll
     for (int b = 0; b < 6; b++) {
       const double w0 = Jc[b] * Jp[0] + Jc[6 + b] * Jp[3];
@@ -2135,11 +2190,11 @@ __device__ __forceinline__ void lm_control(const BADev& p, const lorb_ba_options
 }
 
 // CS: every window of the launch has <= CS_MAX_CAMS cameras, kept in shared memory
-template <bool CS, bool ROBUST = false>
+template <bool CS, bool ROBUST = false, bool WEIGHTED = false>
 __global__ void __launch_bounds__(BA_THREADS, 2)  // latency-bound gathers: two CTAs per SM (ncu: long_scoreboard)
     ba_backsub_kernel(const BADev* __restrict__ probs, lorb_ba_options opt, int fuse_control,
                       int* __restrict__ n_active) {
-  const BADev p = probs[blockIdx.y];
+  const auto p = load_desc<WEIGHTED>(probs, blockIdx.y);
   LMState* st = p.st;
   if (st->done) return;
   __shared__ double red[BA_THREADS / 32];
@@ -2263,11 +2318,11 @@ __global__ void __launch_bounds__(BA_THREADS, 2)  // latency-bound gathers: two 
           const double* rc = CS ? cs + cam * CS_BACKSUB + 51 : camrot_c + CAMROT * cam;
           const double* t = CS ? cs + cam * CS_BACKSUB + 60 : cams_c + 6 * cam + 3;
           const double tt[3] = {t[0], t[1], t[2]};
-          cost_acc += obs_rho<ROBUST>(p, obs_cost(rc, tt, Xc, p.K, (double)uv.x, (double)uv.y));
+          cost_acc += obs_rho<ROBUST>(p, o, obs_cost(rc, tt, Xc, p.K, (double)uv.x, (double)uv.y));
         } else {
           const double* f = p.fixrt + 12 * (size_t)(-1 - cam);
           const double tt[3] = {f[9], f[10], f[11]};
-          cost_acc += obs_rho<ROBUST>(p, obs_cost(f, tt, Xc, p.K, (double)uv.x, (double)uv.y));
+          cost_acc += obs_rho<ROBUST>(p, o, obs_cost(f, tt, Xc, p.K, (double)uv.x, (double)uv.y));
         }
       }
     }
@@ -2307,6 +2362,54 @@ __global__ void ba_control_kernel(const BADev* __restrict__ probs, lorb_ba_optio
   lm_control(p, opt, n_active);
 }
 
+// ---- outlier rounds (lorb_ba_local_rounds_batched); grid (x, window), BADevW descriptors
+
+// Effective weights of the next round: sqrt(w) for an inlier, 0 for an outlier.
+__global__ void __launch_bounds__(256) ba_round_weights_kernel(const BADev* __restrict__ probs) {
+  const BADevW p = load_desc<true>(probs, blockIdx.y);
+  const int n = p.pt_ptr[p.P];
+  for (int o = blockIdx.x * blockDim.x + threadIdx.x; o < n; o += gridDim.x * blockDim.x)
+    p.obs_sw[o] = p.obs_in[o] ? sqrt((double)p.obs_w[o]) : 0.0;
+}
+
+// Classification of every observation of the window at its current parameters (buffer 0, after the
+// solve): chi2 = w |r|^2 (unrobustified), inlier iff chi2 <= th and, with depth_check, the point lies
+// in front of the observing camera.  One thread per point; integer counts, so they do not depend on
+// scheduling.
+__global__ void __launch_bounds__(256)
+    ba_classify_kernel(const BADev* __restrict__ probs, double th, int depth_check) {
+  const BADevW p = load_desc<true>(probs, blockIdx.y);
+  const double* cams = p.cams[0];
+  int cnt = 0;
+  for (int pt = blockIdx.x * blockDim.x + threadIdx.x; pt < p.P; pt += gridDim.x * blockDim.x) {
+    const double X[3] = {p.pts[0][3 * (size_t)pt], p.pts[0][3 * (size_t)pt + 1], p.pts[0][3 * (size_t)pt + 2]};
+    for (int o = p.pt_ptr[pt]; o < p.pt_ptr[pt + 1]; o++) {
+      const int cam = p.obs_cam[o];
+      double R[9], t[3];
+      if (cam >= 0) {
+        cam_rotation(cams + 6 * cam, R, false);
+#pragma unroll
+        for (int a = 0; a < 3; a++) t[a] = cams[6 * cam + 3 + a];
+      } else {
+        const double* f = p.fixrt + 12 * (size_t)(-1 - cam);
+#pragma unroll
+        for (int a = 0; a < 9; a++) R[a] = f[a];
+#pragma unroll
+        for (int a = 0; a < 3; a++) t[a] = f[9 + a];
+      }
+      const double q2 = R[6] * X[0] + R[7] * X[1] + R[8] * X[2] + t[2];
+      const float2 uv = p.obs_uv[o];
+      const double chi2 = (double)p.obs_w[o] * obs_cost(R, t, X, p.K, (double)uv.x, (double)uv.y);
+      const bool in = chi2 <= th && (!depth_check || q2 > 0.0);
+      p.obs_chi2[o] = chi2;
+      p.obs_in[o] = in ? 1 : 0;
+      cnt += in ? 1 : 0;
+    }
+  }
+  cnt = __reduce_add_sync(0xffffffffu, cnt);
+  if ((threadIdx.x & 31) == 0 && cnt) atomicAdd(p.n_in, cnt);
+}
+
 }  // namespace lorb
 
 using namespace lorb;
@@ -2331,6 +2434,9 @@ struct lorb_ba_problem {
   size_t lin_doubles_max = 0, lin_bytes_total = 0;
   double* lin_base = nullptr;
   lorb::LMState* d_states = nullptr;
+  // outlier rounds (lorb_ba_local_rounds_batched): BADevW descriptors and their per-observation arrays
+  std::vector<lorb::BADevW> h_devw;
+  lorb::Buf descs_w, rounds;
 };
 
 namespace lorb {
@@ -2347,6 +2453,19 @@ struct WindowSpec {  // host view of one window's inputs
   const int* fix_pt;
   const float* fix_uv;
   const float* fix_rt;
+  const float* obs_w;  // outlier rounds only: weights [O] / [F] (NULL = 1)
+  const float* fix_w;
+  int obs_base, fix_base;  // outlier rounds only: index of the window's first observation in the caller's arrays
+};
+
+// Host side of an outlier-round solve, filled by problem_build when a rounds entry asks for it:
+// the caller's weights in CSR order and where each caller observation went.
+struct RoundsStage {
+  std::vector<float> w;         // [all windows' O + F], CSR order
+  std::vector<int> obs_slot;    // CSR slot of caller observation obs_base + i
+  std::vector<int> fix_slot;    // CSR slot of caller fixed observation fix_base + i
+  std::vector<size_t> o_obs;    // first CSR slot of each window
+  size_t tot_obs = 0;
 };
 
 static void host_fix_rotation(const float* rt, double* R) {
@@ -2600,7 +2719,7 @@ struct BuildTrace {
 };
 
 static int problem_build(lorb_ba_problem* pb, lorb_ctx* c, const std::vector<WindowSpec>& ws,
-                         const float* K) {
+                         const float* K, RoundsStage* rs = nullptr) {
   const BuildTrace btr;
   pb->ctx = c;
   const int nw = (int)ws.size();
@@ -2654,6 +2773,7 @@ static int problem_build(lorb_ba_problem* pb, lorb_ctx* c, const std::vector<Win
   double* h_pts = reinterpret_cast<double*>(sg + sb_ptr + sb_cam + sb_uv + sb_fix + sb_cams);
   pb->h_cams_stage = h_cams;
   pb->h_pts_stage = h_pts;
+  if (rs) rs->w.assign(std::max<size_t>(tot_obs, 1), 1.0f);
   std::vector<size_t> o_ptr(nw), o_obs(nw), o_fix(nw);
   // large-path work lists (windows with 6C > 96), concatenated over windows
   struct ListOff {
@@ -2744,12 +2864,21 @@ static int problem_build(lorb_ba_problem* pb, lorb_ctx* c, const std::vector<Win
           memcpy(&h_cam[b], W.obs_cam, (size_t)W.O * 4);
           memcpy(&h_uv[b], W.obs_uv, (size_t)W.O * 8);
         }
+        if (rs)
+          for (int i = 0; i < W.O; i++) {
+            rs->obs_slot[W.obs_base + i] = (int)(b + i);
+            rs->w[b + i] = W.obs_w ? W.obs_w[i] : 1.0f;
+          }
       } else {
         fill.assign(ptr, ptr + W.P);
         for (int i = 0; i < W.O; i++) {
           const int d = fill[W.obs_pt[i]]++;
           h_cam[b + d] = W.obs_cam[i];
           h_uv[b + d] = make_float2(W.obs_uv[2 * i], W.obs_uv[2 * i + 1]);
+          if (rs) {
+            rs->obs_slot[W.obs_base + i] = (int)(b + d);
+            rs->w[b + d] = W.obs_w ? W.obs_w[i] : 1.0f;
+          }
         }
       }
       for (int i = 0; i < W.F; i++) {
@@ -2757,6 +2886,10 @@ static int problem_build(lorb_ba_problem* pb, lorb_ctx* c, const std::vector<Win
         h_cam[b + d] = -1 - i;
         h_uv[b + d] = make_float2(W.fix_uv[2 * i], W.fix_uv[2 * i + 1]);
         host_fix_rotation(W.fix_rt + 6 * (size_t)i, &h_fix[12 * (f + i)]);
+        if (rs) {
+          rs->fix_slot[W.fix_base + i] = (int)(b + d);
+          rs->w[b + d] = W.fix_w ? W.fix_w[i] : 1.0f;
+        }
       }
       if (6 * W.C <= DENSE_N) {
         // the atomic-free dense path stores (point, camera) tiles: needs unique pairs
@@ -2793,6 +2926,10 @@ static int problem_build(lorb_ba_problem* pb, lorb_ctx* c, const std::vector<Win
       if (W.P) memcpy(&h_pts[3 * (size_t)pb->h_pt_off[w]], W.pts, (size_t)W.P * 24);
     }
     LORB_REQUIRE(!bad_obs, "observation index out of range");
+    if (rs) {
+      rs->o_obs = o_obs;
+      rs->tot_obs = tot_obs;
+    }
     LORB_REQUIRE(!bad_fix, "fixed observation point out of range");
     pb->has_dup = dup_any != 0;
   }
@@ -3031,8 +3168,10 @@ static int run_cholesky(lorb_ba_problem* pb) {
   return LORB_OK;
 }
 
+// round_loss: a round of an outlier-round solve under that loss (the WEIGHTED instantiations, with
+// the BADevW descriptors of the problem); NULL: a plain solve under the ctx's loss.
 static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int sharded,
-                         lorb_ba_summary* sums) {
+                         lorb_ba_summary* sums, const lorb_ba_loss* round_loss = nullptr) {
   lorb_ctx* c = pb->ctx;
   const BADev* dp = pb->descs.as<BADev>();
   const BADev& d0 = pb->h_dev[0];
@@ -3051,8 +3190,9 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
       LORB_CUDA_TRY(cudaMemcpyAsync(pb->descs.p, &h0, sizeof(BADev), cudaMemcpyHostToDevice, c->stream));
     }
   }
-  // the robust loss is the ctx's at solve time: every window's descriptor carries it
-  const lorb_ba_loss loss = c->ba_loss;
+  // the robust loss is the ctx's at solve time (a round's own one): every window's descriptor carries it
+  const lorb_ba_loss loss = round_loss ? *round_loss : c->ba_loss;
+  const bool weighted = round_loss != nullptr;
   const bool robust = loss.kind != LORB_LOSS_TRIVIAL;
   {
     bool changed = false;
@@ -3065,8 +3205,19 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
       LORB_CUDA_TRY(cudaMemcpyAsync(pb->descs.p, pb->h_dev.data(), sizeof(BADev) * (size_t)nw,
                                     cudaMemcpyHostToDevice, c->stream));
   }
-  // kernel instantiation for the loss: ROBUST = false is plain least squares, unchanged
-#define LORB_BA_K(K_, ...) (robust ? K_<__VA_ARGS__, true> : K_<__VA_ARGS__, false>)
+  if (weighted) {
+    LORB_REQUIRE(!sharded && pb->h_devw.size() == (size_t)nw, "outlier rounds: descriptors (internal)");
+    for (int w = 0; w < nw; w++) static_cast<BADev&>(pb->h_devw[w]) = pb->h_dev[w];
+    LORB_CUDA_TRY(cudaMemcpyAsync(pb->descs_w.p, pb->h_devw.data(), sizeof(BADevW) * (size_t)nw,
+                                  cudaMemcpyHostToDevice, c->stream));
+  }
+  // kernels that evaluate observations read their descriptors through dpk
+  const BADev* dpk = weighted ? reinterpret_cast<const BADev*>(pb->descs_w.p) : dp;
+  // kernel instantiation for the loss: ROBUST = false is plain least squares, unchanged; an outlier
+  // round runs the WEIGHTED form of the robust code, with the trivial loss in its plain rounds
+#define LORB_BA_K(K_, ...) \
+  (weighted ? K_<__VA_ARGS__, true, true> : robust ? K_<__VA_ARGS__, true> : K_<__VA_ARGS__, false>)
+#define LORB_BA_K0(K_) (weighted ? K_<true, true> : robust ? K_<true> : K_<false>)
   const int gx_pts = std::max(1, std::min((pb->maxP + 31) / 32, std::max(1, c->sm_count * 8 / nw)));
   const dim3 grid_pts(gx_pts, nw);
   // back-substitution with the cameras in shared memory: two CTAs per SM must fit (C <= 203); a CTA
@@ -3134,16 +3285,16 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
   auto launch_build = [&](bool full, int force) -> int {
     const size_t sm = full ? smem_build_full : smem_build_init;
 #define LORB_BUILD(FULL_, ACC_) \
-  LORB_LAUNCH(c, LORB_BA_K(ba_build_kernel, FULL_, ACC_), grid_pts, BA_THREADS, sm, dp, opt, force)
+  LORB_LAUNCH(c, LORB_BA_K(ba_build_kernel, FULL_, ACC_), grid_pts, BA_THREADS, sm, dpk, opt, force)
     if (acc_mode == 2) {
-      if (full) LORB_LAUNCH(c, LORB_BA_K(ba_build_dense_kernel, true), grid_dense, DP_THREADS, DP_SMEM_DOUBLES * 8, dp, opt, force);
-      else      LORB_LAUNCH(c, LORB_BA_K(ba_build_dense_kernel, false), grid_dense, DP_THREADS, DP_SMEM_DOUBLES * 8, dp, opt, force);
+      if (full) LORB_LAUNCH(c, LORB_BA_K(ba_build_dense_kernel, true), grid_dense, DP_THREADS, DP_SMEM_DOUBLES * 8, dpk, opt, force);
+      else      LORB_LAUNCH(c, LORB_BA_K(ba_build_dense_kernel, false), grid_dense, DP_THREADS, DP_SMEM_DOUBLES * 8, dpk, opt, force);
     } else if (acc_mode == 1) {
       if (full) LORB_BUILD(true, 1); else LORB_BUILD(false, 1);
     } else {
       // large path: point side, then camera side and Schur products from the work lists
-      if (full) LORB_LAUNCH(c, LORB_BA_K(ba_build_kernel, true, 3), grid_pts, BA_THREADS, 0, dp, opt, force);
-      else      LORB_LAUNCH(c, LORB_BA_K(ba_build_kernel, false, 3), grid_pts, BA_THREADS, 0, dp, opt, force);
+      if (full) LORB_LAUNCH(c, LORB_BA_K(ba_build_kernel, true, 3), grid_pts, BA_THREADS, 0, dpk, opt, force);
+      else      LORB_LAUNCH(c, LORB_BA_K(ba_build_kernel, false, 3), grid_pts, BA_THREADS, 0, dpk, opt, force);
       // camera rows (H_cc, g_c, Schur rhs) and Schur pairs (S) both need only the point side and write
       // disjoint outputs; both are latency-bound gathers, so the camera rows run on a side stream
       // beside the (six times longer) pair pass
@@ -3155,19 +3306,16 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
         }
         LORB_CUDA_TRY(cudaEventRecord(c->ba_ev[0], c->stream));
         LORB_CUDA_TRY(cudaStreamWaitEvent(c->ba_stream2, c->ba_ev[0], 0));
-        (robust ? ba_cam_rows_kernel<true> : ba_cam_rows_kernel<false>)
-            <<<dim3((pb->max_cam_items + 7) / 8, nw), 256, 0, c->ba_stream2>>>(dp, 1, force);
+        LORB_BA_K0(ba_cam_rows_kernel)<<<dim3((pb->max_cam_items + 7) / 8, nw), 256, 0, c->ba_stream2>>>(dpk, 1, force);
         c->launches++;
         LORB_CUDA_TRY(cudaGetLastError());
         LORB_CUDA_TRY(cudaEventRecord(c->ba_ev[1], c->ba_stream2));
       } else if (pb->max_cam_items > 0) {
-        LORB_LAUNCH(c, (robust ? ba_cam_rows_kernel<true> : ba_cam_rows_kernel<false>),
-                    dim3((pb->max_cam_items + 7) / 8, nw), 256, 0, dp,
+        LORB_LAUNCH(c, LORB_BA_K0(ba_cam_rows_kernel), dim3((pb->max_cam_items + 7) / 8, nw), 256, 0, dpk,
                     full ? 1 : 0, force);
       }
       if (full && pb->max_pair_items > 0)
-        LORB_LAUNCH(c, (robust ? ba_schur_pairs_kernel<true> : ba_schur_pairs_kernel<false>),
-                    dim3((pb->max_pair_items + 7) / 8, nw), 256, 0, dp);
+        LORB_LAUNCH(c, LORB_BA_K0(ba_schur_pairs_kernel), dim3((pb->max_pair_items + 7) / 8, nw), 256, 0, dpk);
       if (side) LORB_CUDA_TRY(cudaStreamWaitEvent(c->stream, c->ba_ev[1], 0));
     }
 #undef LORB_BUILD
@@ -3212,10 +3360,10 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
     prof_end(c, 2);
     prof_begin(c, 1);
     if (backsub_cs)
-      LORB_LAUNCH(c, LORB_BA_K(ba_backsub_kernel, true), grid_backsub, BA_THREADS, backsub_smem, dp, opt, fuse_control,
+      LORB_LAUNCH(c, LORB_BA_K(ba_backsub_kernel, true), grid_backsub, BA_THREADS, backsub_smem, dpk, opt, fuse_control,
                   d_active);
     else
-      LORB_LAUNCH(c, LORB_BA_K(ba_backsub_kernel, false), grid_pts, BA_THREADS, 0, dp, opt, fuse_control, d_active);
+      LORB_LAUNCH(c, LORB_BA_K(ba_backsub_kernel, false), grid_pts, BA_THREADS, 0, dpk, opt, fuse_control, d_active);
     prof_end(c, 1);
     if (sharded) {
       prof_begin(c, 4);
@@ -3272,6 +3420,7 @@ static int problem_solve(lorb_ba_problem* pb, const lorb_ba_options* optp, int s
   LORB_CUDA_TRY(cudaStreamSynchronize(s));
   return LORB_OK;
 #undef LORB_BA_K
+#undef LORB_BA_K0
 }
 
 // The host-buffer entry points (lorb_ba_local, lorb_ba_local_batched) reuse one
@@ -3298,6 +3447,8 @@ static void problem_free(lorb_ba_problem* pb) {
   pb->list_scratch2.release();
   pb->hstate.release();
   pb->counter.release();
+  pb->descs_w.release();
+  pb->rounds.release();
   delete pb;
 }
 
@@ -3591,6 +3742,157 @@ int lorb_ba_local_batched(lorb_ctx* c, int n_windows, const int* cam_off, double
   LORB_TRY(problem_reset(pb));
   LORB_TRY(problem_solve(pb, opt, 0, summaries));
   return lorb_ba_problem_download(pb, cams, pts);
+}
+
+void lorb_ba_default_local_rounds(lorb_ba_local_rounds* r, lorb_ba_options* opt2) {
+  if (r) {
+    r->n_rounds = 2;
+    r->robust_rounds = 1;
+    r->chi2 = 5.991;
+    r->depth_check = 1;
+    r->reserved = 0;
+  }
+  if (opt2) {
+    lorb_ba_default_options(&opt2[0]);
+    lorb_ba_default_options(&opt2[1]);
+    opt2[0].max_num_iterations = 5;
+    opt2[1].max_num_iterations = 10;
+  }
+}
+
+static bool weights_ok(const float* w, int lo, int hi) {
+  if (!w) return true;
+  for (int i = lo; i < hi; i++)
+    if (!(std::isfinite(w[i]) && w[i] > 0.0f)) return false;
+  return true;
+}
+
+int lorb_ba_local_rounds_batched(lorb_ctx* c, int n_windows, const int* cam_off, double* cams, const int* pt_off,
+                                 double* pts, const int* obs_off, const int* obs_cam, const int* obs_pt,
+                                 const float* obs_uv, const float* obs_w, const int* fix_off, const int* fix_pt,
+                                 const float* fix_uv, const float* fix_rt, const float* fix_w, const float* K,
+                                 const lorb_ba_local_rounds* rounds, const lorb_ba_options* opt,
+                                 uint8_t* obs_inlier, double* obs_chi2, uint8_t* fix_inlier, double* fix_chi2,
+                                 int* n_inliers, lorb_ba_summary* summaries) {
+  LORB_REQUIRE(c && opt && K && rounds, "ctx / options / K / rounds");
+  LORB_REQUIRE(rounds->n_rounds >= 1 && rounds->n_rounds <= 16, "rounds->n_rounds (1..16)");
+  LORB_REQUIRE(rounds->robust_rounds >= 0 && rounds->robust_rounds <= rounds->n_rounds,
+               "rounds->robust_rounds (0..n_rounds)");
+  LORB_REQUIRE(std::isfinite(rounds->chi2) && rounds->chi2 > 0.0, "rounds->chi2 (finite, > 0)");
+  LORB_REQUIRE(rounds->depth_check == 0 || rounds->depth_check == 1, "rounds->depth_check (0 / 1)");
+  LORB_REQUIRE(n_windows >= 0, "n_windows");
+  if (n_windows == 0) return LORB_OK;
+  LORB_REQUIRE(cam_off && pt_off && obs_off && cams && n_inliers, "window offsets / cams / n_inliers");
+  for (int w = 0; w < n_windows; w++) {
+    LORB_REQUIRE(cam_off[w + 1] > cam_off[w] && pt_off[w + 1] >= pt_off[w] && obs_off[w + 1] >= obs_off[w] &&
+                     (!fix_off || fix_off[w + 1] >= fix_off[w]),
+                 "window sizes");
+  }
+  const int o0 = obs_off[0], o1 = obs_off[n_windows];
+  const int f0 = fix_off ? fix_off[0] : 0, f1 = fix_off ? fix_off[n_windows] : 0;
+  LORB_REQUIRE(o1 == o0 || obs_inlier, "obs_inlier");
+  LORB_REQUIRE(f1 == f0 || fix_inlier, "fix_inlier");
+  LORB_REQUIRE(weights_ok(obs_w, o0, o1), "obs_w (finite, > 0)");
+  LORB_REQUIRE(f1 == f0 || weights_ok(fix_w, f0, f1), "fix_w (finite, > 0)");
+  LORB_CUDA_TRY(cudaSetDevice(c->device));
+  std::vector<WindowSpec> ws;
+  LORB_TRY(batched_specs(ws, n_windows, cam_off, cams, pt_off, pts, obs_off, obs_cam, obs_pt, obs_uv,
+                         fix_off, fix_pt, fix_uv, fix_rt));
+  for (int w = 0; w < n_windows; w++) {
+    WindowSpec& W = ws[w];
+    W.obs_base = obs_off[w] - o0;
+    W.fix_base = fix_off ? fix_off[w] - f0 : 0;
+    W.obs_w = obs_w ? obs_w + obs_off[w] : nullptr;
+    W.fix_w = fix_w && fix_off ? fix_w + fix_off[w] : nullptr;
+  }
+  lorb_ba_problem* pb = cached_problem(c);
+  if (!pb) return LORB_ERR_NOMEM;
+  RoundsStage rs;
+  rs.obs_slot.assign((size_t)(o1 - o0), 0);
+  rs.fix_slot.assign((size_t)(f1 - f0), 0);
+  LORB_TRY(problem_build(pb, c, ws, K, &rs));
+  LORB_TRY(problem_reset(pb));
+  // per-observation arrays of the rounds: sqrt of the effective weight | weight | flag | chi2 | counts
+  const int nw = n_windows, R = rounds->n_rounds;
+  const size_t OT = std::max<size_t>(rs.tot_obs, 1);
+  const size_t b_sw = al(OT * 8), b_w = al(OT * 4), b_in = al(OT), b_chi = al(OT * 8), b_n = al((size_t)nw * 4);
+  LORB_TRY(pb->rounds.reserve(b_sw + b_w + b_in + b_chi + b_n));
+  LORB_TRY(pb->descs_w.reserve(sizeof(BADevW) * (size_t)nw));
+  uint8_t* q = pb->rounds.as<uint8_t>();
+  double* d_sw = reinterpret_cast<double*>(q);
+  float* d_w = reinterpret_cast<float*>(q + b_sw);
+  uint8_t* d_in = q + b_sw + b_w;
+  double* d_chi = reinterpret_cast<double*>(q + b_sw + b_w + b_in);
+  int* d_n = reinterpret_cast<int*>(q + b_sw + b_w + b_in + b_chi);
+  pb->h_devw.resize((size_t)nw);
+  for (int w = 0; w < nw; w++) {
+    BADevW& d = pb->h_devw[w];
+    static_cast<BADev&>(d) = pb->h_dev[w];
+    d.obs_sw = d_sw + rs.o_obs[w];
+    d.obs_w = d_w + rs.o_obs[w];
+    d.obs_in = d_in + rs.o_obs[w];
+    d.obs_chi2 = d_chi + rs.o_obs[w];
+    d.n_in = d_n + w;
+  }
+  cudaStream_t s = c->stream;
+  const BADev* dpw = reinterpret_cast<const BADev*>(pb->descs_w.p);
+  LORB_CUDA_TRY(cudaMemcpyAsync(pb->descs_w.p, pb->h_devw.data(), sizeof(BADevW) * (size_t)nw,
+                                cudaMemcpyHostToDevice, s));
+  LORB_CUDA_TRY(cudaMemcpyAsync(d_w, rs.w.data(), rs.tot_obs * 4, cudaMemcpyHostToDevice, s));
+  LORB_CUDA_TRY(cudaMemsetAsync(d_in, 1, rs.tot_obs, s));  // round 0 solves over every observation
+  int max_obs = 0, max_p = 0;
+  for (const WindowSpec& W : ws) {
+    max_obs = std::max(max_obs, W.O + W.F);
+    max_p = std::max(max_p, W.P);
+  }
+  const dim3 grid_obs(std::max(1, std::min((max_obs + 255) / 256, std::max(1, c->sm_count * 4 / nw))), nw);
+  const dim3 grid_pt(std::max(1, std::min((max_p + 255) / 256, std::max(1, c->sm_count * 4 / nw))), nw);
+  std::vector<lorb_ba_summary> sr((size_t)nw);
+  const lorb_ba_loss plain = {LORB_LOSS_TRIVIAL, 0, 1.0};
+  for (int r = 0; r < R; r++) {
+    const lorb_ba_loss loss = r < rounds->robust_rounds ? c->ba_loss : plain;
+    LORB_LAUNCH(c, ba_round_weights_kernel, grid_obs, 256, 0, dpw);
+    LORB_TRY(problem_solve(pb, &opt[r], 0, sr.data(), &loss));
+    LORB_CUDA_TRY(cudaMemsetAsync(d_n, 0, (size_t)nw * 4, s));
+    LORB_LAUNCH(c, ba_classify_kernel, grid_pt, 256, 0, dpw, rounds->chi2, rounds->depth_check);
+    if (summaries)
+      for (int w = 0; w < nw; w++) summaries[(size_t)w * R + r] = sr[w];
+  }
+  std::vector<uint8_t> h_in(rs.tot_obs);
+  std::vector<double> h_chi(rs.tot_obs);
+  LORB_CUDA_TRY(cudaMemcpyAsync(h_in.data(), d_in, rs.tot_obs, cudaMemcpyDeviceToHost, s));
+  LORB_CUDA_TRY(cudaMemcpyAsync(h_chi.data(), d_chi, rs.tot_obs * 8, cudaMemcpyDeviceToHost, s));
+  LORB_CUDA_TRY(cudaMemcpyAsync(n_inliers, d_n, (size_t)nw * 4, cudaMemcpyDeviceToHost, s));
+  LORB_TRY(lorb_ba_problem_download(pb, cams, pts));  // synchronises the stream
+  // flags and chi-square values back in the caller's order
+  for (int i = 0; i < o1 - o0; i++) {
+    const int k = rs.obs_slot[i];
+    obs_inlier[o0 + i] = h_in[k];
+    if (obs_chi2) obs_chi2[o0 + i] = h_chi[k];
+  }
+  for (int i = 0; i < f1 - f0; i++) {
+    const int k = rs.fix_slot[i];
+    fix_inlier[f0 + i] = h_in[k];
+    if (fix_chi2) fix_chi2[f0 + i] = h_chi[k];
+  }
+  return LORB_OK;
+}
+
+int lorb_ba_local_rounds_single(lorb_ctx* c, int C, double* cams, int P, double* pts, int O, const int* obs_cam,
+                                const int* obs_pt, const float* obs_uv, const float* obs_w, int F,
+                                const int* fix_pt, const float* fix_uv, const float* fix_rt, const float* fix_w,
+                                const float* K, const lorb_ba_local_rounds* rounds, const lorb_ba_options* opt,
+                                uint8_t* obs_inlier, double* obs_chi2, uint8_t* fix_inlier, double* fix_chi2,
+                                int* n_inliers, lorb_ba_summary* summaries) {
+  LORB_REQUIRE(c && opt && K, "ctx / options / K");
+  LORB_REQUIRE(C > 0 && P >= 0 && O >= 0 && F >= 0, "sizes");
+  LORB_REQUIRE(cams && (P == 0 || pts), "parameters");
+  LORB_REQUIRE(O == 0 || (obs_cam && obs_pt && obs_uv), "observations");
+  LORB_REQUIRE(F == 0 || (fix_pt && fix_uv && fix_rt), "fixed observations");
+  const int cam_off[2] = {0, C}, pt_off[2] = {0, P}, obs_off[2] = {0, O}, fix_off[2] = {0, F};
+  return lorb_ba_local_rounds_batched(c, 1, cam_off, cams, pt_off, pts, obs_off, obs_cam, obs_pt, obs_uv, obs_w,
+                                      fix_off, fix_pt, fix_uv, fix_rt, fix_w, K, rounds, opt, obs_inlier, obs_chi2,
+                                      fix_inlier, fix_chi2, n_inliers, summaries);
 }
 
 /* Team size of the host-side staging loops (OpenMP) of the calling thread.  A launcher such as

@@ -43,6 +43,11 @@ struct LocalBAWindow
 	std::vector<float> obs_uv;                        // [O][2]
 	std::vector<int> fix_pt;                          // [F]
 	std::vector<float> fix_uv, fix_rt;                // [F][2], [F][6]
+	// the keypoint behind each record: in-window observation i is keypoint obs_kp[i] of
+	// frames[obs_cam[i]]; fixed observation i is keypoint fix_kp[i] of fix_frame[i]
+	std::vector<int> obs_kp;                          // [O]
+	std::vector<Simple_ORB_SLAM::Frame*> fix_frame;   // [F]
+	std::vector<int> fix_kp;                          // [F]
 	void clear();
 };
 
@@ -61,6 +66,16 @@ public:
 	void Assemble(Simple_ORB_SLAM::Frame* pCurrFrame, LocalBAWindow& w);
 	// BA::LocalPoseOptimization(pCurrFrame) with the problem taken from the index.
 	void Optimize(Simple_ORB_SLAM::Frame* pCurrFrame);
+	// ORB-SLAM2's Optimizer::LocalBundleAdjustment over the same problem (lorb_ba_local_rounds_single
+	// with lorb_ba_default_local_rounds: 5 iterations under Huber sqrt(chi2), then 10 plain ones over the
+	// inliers; every observation weighted by 1 / sigma^2 of its keypoint's octave, read from the
+	// observing frame's mvScaleFactors / mvKeysUn).  The ctx's loss is put back afterwards.  Writes the
+	// floats back as Optimize does, then erases every observation flagged outlier (chi^2 > 5.991 or
+	// not in front of its camera): the frame's mvpMapPoints[kp] becomes NULL, the point's mnObs drops
+	// by one and the index forgets the observation, so no later Assemble sees it.  The map point's own
+	// observation map is private in the reference and is left alone.  Returns the number of erased
+	// observations.
+	int OptimizeRejectingOutliers(Simple_ORB_SLAM::Frame* pCurrFrame);
 
 	size_t NumFrames() const { return mFrames.size(); }
 	size_t NumPoints() const { return mPoints.size(); }
@@ -71,6 +86,7 @@ private:
 	int FrameId(Simple_ORB_SLAM::Frame* pF);
 	int PointId(Simple_ORB_SLAM::MapPoint* pMP);
 	void Record(int pid, int fid, int kp);
+	void Forget(int pid, int fid);
 
 	std::unordered_map<Simple_ORB_SLAM::Frame*, int> mFrameIds;
 	std::unordered_map<Simple_ORB_SLAM::MapPoint*, int> mPointIds;

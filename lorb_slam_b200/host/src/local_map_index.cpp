@@ -3,6 +3,8 @@
 #include "../include/local_map_index.h"
 
 #include <algorithm>
+#include <cmath>
+#include <cstdint>
 #include <functional>
 
 #include "lorb_host.h"
@@ -17,6 +19,7 @@ void LocalBAWindow::clear()
 	frames.clear(); points.clear(); cams.clear(); pts.clear();
 	obs_cam.clear(); obs_pt.clear(); obs_uv.clear();
 	fix_pt.clear(); fix_uv.clear(); fix_rt.clear();
+	obs_kp.clear(); fix_frame.clear(); fix_kp.clear();
 }
 
 int LocalMapIndex::FrameId(Frame* pF)
@@ -50,6 +53,24 @@ void LocalMapIndex::Record(int pid, int fid, int kp)
 	Obs o; o.frame = fid; o.kp = kp;
 	v.insert(v.begin() + k, o);
 	mnObservations++;
+}
+
+// The observation of point pid by frame fid leaves the index: its per-point record and the frame's
+// slot entry of that point.
+void LocalMapIndex::Forget(int pid, int fid)
+{
+	std::vector<Obs>& v = mPointObs[pid];
+	for(size_t k=0; k<v.size(); k++)
+		if(v[k].frame == fid)
+		{
+			v.erase(v.begin() + k);
+			mnObservations--;
+			break;
+		}
+	std::vector<int>& slots = mFramePoints[fid];
+	std::vector<int>::iterator it = std::find(slots.begin(), slots.end(), pid);
+	if(it != slots.end())
+		slots.erase(it);
 }
 
 int LocalMapIndex::PointId(MapPoint* pMP)
@@ -177,6 +198,7 @@ void LocalMapIndex::Assemble(Frame* pCurrFrame, LocalBAWindow& w)
 				w.obs_cam.push_back(mFrameWindowIdx[v[k].frame]);
 				w.obs_pt.push_back((int)i);
 				w.obs_uv.push_back(kp2d.x); w.obs_uv.push_back(kp2d.y);
+				w.obs_kp.push_back(v[k].kp);
 			}
 			else
 			{
@@ -184,9 +206,34 @@ void LocalMapIndex::Assemble(Frame* pCurrFrame, LocalBAWindow& w)
 				w.fix_uv.push_back(kp2d.x); w.fix_uv.push_back(kp2d.y);
 				for(int a=0; a<3; a++) w.fix_rt.push_back(pF->mRvec.at<float>(a));
 				for(int a=0; a<3; a++) w.fix_rt.push_back(pF->mTvec.at<float>(a));
+				w.fix_frame.push_back(pF);
+				w.fix_kp.push_back(v[k].kp);
 			}
 		}
 	}
+}
+
+// float write-back of a solved window (src/bundle_adjust.cpp:317-329)
+static void WriteBack(const LocalBAWindow& w)
+{
+	for(size_t i=0; i<w.frames.size(); i++)
+	{
+		cv::Mat R(3, 1, CV_32F), T(3, 1, CV_32F);
+		for(int k=0; k<3; k++)
+		{
+			R.at<float>(k) = (float)w.cams[6*i+k];
+			T.at<float>(k) = (float)w.cams[6*i+3+k];
+		}
+		w.frames[i]->SetPose(T, R);
+	}
+	for(size_t i=0; i<w.points.size(); i++)
+		w.points[i]->SetWorldPos(cv::Point3f((float)w.pts[3*i], (float)w.pts[3*i+1], (float)w.pts[3*i+2]));
+}
+
+static float InvSigma2(Frame* pF, int kp)
+{
+	const float s = pF->mvScaleFactors[pF->mvKeysUn[kp].octave];
+	return 1.0f / (s * s);
 }
 
 void LocalMapIndex::Optimize(Frame* pCurrFrame)
@@ -202,19 +249,52 @@ void LocalMapIndex::Optimize(Frame* pCurrFrame)
 	                             w.pts.data(), (int)w.obs_cam.size(), w.obs_cam.data(), w.obs_pt.data(),
 	                             w.obs_uv.data(), (int)w.fix_pt.size(), w.fix_pt.data(), w.fix_uv.data(),
 	                             w.fix_rt.data(), K, &opt, &summary));
-	// write back as float (:317-329)
-	for(size_t i=0; i<w.frames.size(); i++)
+	WriteBack(w);
+}
+
+int LocalMapIndex::OptimizeRejectingOutliers(Frame* pCurrFrame)
+{
+	LocalBAWindow& w = mWindow;
+	Assemble(pCurrFrame, w);
+	const Camera* cam = pCurrFrame->mpCamera;
+	const float K[4] = {cam->fx, cam->fy, cam->cx, cam->cy};
+	const int O = (int)w.obs_cam.size(), F = (int)w.fix_pt.size();
+	std::vector<float> obs_w(O), fix_w(F);
+	for(int i=0; i<O; i++)
+		obs_w[i] = InvSigma2(w.frames[w.obs_cam[i]], w.obs_kp[i]);
+	for(int i=0; i<F; i++)
+		fix_w[i] = InvSigma2(w.fix_frame[i], w.fix_kp[i]);
+	lorb_ba_local_rounds rounds;
+	lorb_ba_options opt[2];
+	lorb_ba_default_local_rounds(&rounds, opt);
+	std::vector<uint8_t> obs_in(O), fix_in(F);
+	int n_in = 0;
+	lorb_ctx* c = ctx();
+	lorb_ba_loss prev, huber = {LORB_LOSS_HUBER, 0, std::sqrt(rounds.chi2)};
+	LORB_HOST_CALL(lorb_ba_get_loss(c, &prev));
+	LORB_HOST_CALL(lorb_ba_set_loss(c, &huber));
+	const int rc = lorb_ba_local_rounds_single(c, (int)w.frames.size(), w.cams.data(), (int)w.points.size(),
+	                                           w.pts.data(), O, w.obs_cam.data(), w.obs_pt.data(), w.obs_uv.data(),
+	                                           obs_w.data(), F, w.fix_pt.data(), w.fix_uv.data(), w.fix_rt.data(),
+	                                           fix_w.data(), K, &rounds, opt, obs_in.data(), NULL, fix_in.data(),
+	                                           NULL, &n_in, NULL);
+	LORB_HOST_CALL(lorb_ba_set_loss(c, &prev));
+	if(rc != LORB_OK) die("lorb_ba_local_rounds_single", rc);
+	WriteBack(w);
+	int n_erased = 0;
+	for(int i=0; i<O+F; i++)
 	{
-		cv::Mat R(3, 1, CV_32F), T(3, 1, CV_32F);
-		for(int k=0; k<3; k++)
-		{
-			R.at<float>(k) = (float)w.cams[6*i+k];
-			T.at<float>(k) = (float)w.cams[6*i+3+k];
-		}
-		w.frames[i]->SetPose(T, R);
+		if(i < O ? obs_in[i] : fix_in[i-O])
+			continue;
+		Frame* pF = i < O ? w.frames[w.obs_cam[i]] : w.fix_frame[i-O];
+		const int kp = i < O ? w.obs_kp[i] : w.fix_kp[i-O];
+		MapPoint* pMP = w.points[i < O ? w.obs_pt[i] : w.fix_pt[i-O]];
+		pF->mvpMapPoints[kp] = NULL;
+		pMP->mnObs--;
+		Forget(PointId(pMP), FrameId(pF));
+		n_erased++;
 	}
-	for(size_t i=0; i<w.points.size(); i++)
-		w.points[i]->SetWorldPos(cv::Point3f((float)w.pts[3*i], (float)w.pts[3*i+1], (float)w.pts[3*i+2]));
+	return n_erased;
 }
 
 }

@@ -418,6 +418,79 @@ int harness_local_mapping(int n_kf, const float* kf_rt, const int* kf_off, const
 	return n_ba;
 }
 
+// The mapper's loop with outlier removal: as harness_local_mapping's world A, but the local BA of every
+// new keyframe from `first_ba` on is LocalMapIndex::OptimizeRejectingOutliers (reject = 1) or Optimize
+// (reject = 0).  Slot s carries the ORB octave slot_oct[s]; every frame has the 8-level 1.2 pyramid.
+// Outputs: final float poses / points, per slot whether mvpMapPoints ended NULL (slot_null) and whether
+// the final Assemble of the last keyframe still holds that observation (slot_assembled), mnObs per point.
+// Returns the number of erased observations.
+int harness_local_mapping_rejecting(int n_kf, const float* kf_rt, const int* kf_off, const int* slot_pt,
+                                    const float* slot_uv, const int* slot_oct, const int* cov_off,
+                                    const int* cov_idx, int P, const float* pts, const float* K4, int first_ba,
+                                    int reject, float* out_cams, float* out_pts, uint8_t* slot_null,
+                                    uint8_t* slot_assembled, int* mnobs)
+{
+	Camera cam;
+	cam.fx = K4[0]; cam.fy = K4[1]; cam.cx = K4[2]; cam.cy = K4[3];
+	std::vector<Frame> frames(n_kf);
+	std::vector<MapPoint> mps(P);
+	for(int p=0;p<P;p++) mps[p].mWorldPos = cv::Point3f(pts[3*p], pts[3*p+1], pts[3*p+2]);
+	lorb_host::LocalMapIndex index;
+	int n_erased = 0;
+	for(int k=0; k<n_kf; k++)
+	{
+		Frame& F = frames[k];
+		F.mpCamera = &cam;
+		for(int l=0; l<8; l++) F.mvScaleFactors.push_back(std::pow(1.2f, (float)l));
+		cv::Mat R(3,1,CV_32F), T(3,1,CV_32F);
+		for(int a=0;a<3;a++) { R.at<float>(a) = kf_rt[6*k+a]; T.at<float>(a) = kf_rt[6*k+3+a]; }
+		F.SetPose(T, R);
+		for(int s=kf_off[k]; s<kf_off[k+1]; s++)
+		{
+			cv::KeyPoint kp;
+			kp.pt = cv::Point2f(slot_uv[2*s], slot_uv[2*s+1]);
+			kp.octave = slot_oct[s];
+			F.mvKeysUn.push_back(kp);
+			F.mvpMapPoints.push_back(slot_pt[s] >= 0 ? &mps[slot_pt[s]] : static_cast<MapPoint*>(NULL));
+		}
+		F.mnMapPoints = F.mvKeysUn.size();
+		for(int c=cov_off[k]; c<cov_off[k+1]; c++) F.mvpOrderedKeyFrames.push_back(&frames[cov_idx[c]]);
+		index.InsertKeyFrame(&F);
+		if(k < first_ba)
+			continue;
+		if(reject)
+			n_erased += index.OptimizeRejectingOutliers(&F);
+		else
+			index.Optimize(&F);
+	}
+	for(int k=0;k<n_kf;k++)
+	{
+		for(int a=0;a<3;a++)
+		{
+			out_cams[6*k+a] = frames[k].mRvec.at<float>(a);
+			out_cams[6*k+3+a] = frames[k].mTvec.at<float>(a);
+		}
+		for(int s=kf_off[k]; s<kf_off[k+1]; s++)
+		{
+			slot_null[s] = slot_pt[s] >= 0 && frames[k].mvpMapPoints[s - kf_off[k]] == NULL;
+			slot_assembled[s] = 0;
+		}
+	}
+	for(int p=0;p<P;p++)
+	{
+		const cv::Point3f q = mps[p].GetPos();
+		out_pts[3*p] = q.x; out_pts[3*p+1] = q.y; out_pts[3*p+2] = q.z;
+		mnobs[p] = (int)mps[p].mnObs;
+	}
+	lorb_host::LocalBAWindow w;
+	index.Assemble(&frames[n_kf-1], w);
+	for(size_t i=0; i<w.obs_kp.size(); i++)
+		slot_assembled[kf_off[w.frames[w.obs_cam[i]] - &frames[0]] + w.obs_kp[i]] = 1;
+	for(size_t i=0; i<w.fix_kp.size(); i++)
+		slot_assembled[kf_off[w.fix_frame[i] - &frames[0]] + w.fix_kp[i]] = 1;
+	return n_erased;
+}
+
 // LocalMapIndex on its own (host logic only, no device call): insert the keyframes, then assemble the
 // local-BA problem of keyframe `k_ba` and hand its index arrays back.  Same inputs as
 // harness_local_mapping; bad_kf / bad_pt flag frames / points whose IsBad() is true.
