@@ -17,19 +17,19 @@ LOSS_NAME = os.environ.get("LORB_SOAK_LOSS", "")
 LOSS = None
 if LOSS_NAME:
     sys.path.insert(0, "tests")
+    import oracle_ext  # noqa: E402
     import robust_cases  # noqa: E402
-    import robust_ref  # noqa: E402
     LOSS = (robust_cases.LOSSES[LOSS_NAME], float(os.environ.get("LORB_SOAK_LOSS_SCALE", 2.0)))
     _orng = np.random.default_rng(5)  # outliers from a stream of their own: the problem draws stay as they are
 
 
 def oracle_local(pb, opt):
-    return ref.ba_local(pb, opt) if LOSS is None else robust_ref.ba_local(pb, opt, loss=LOSS)
+    return ref.ba_local(pb, opt) if LOSS is None else oracle_ext.ba_local(pb, opt, loss=LOSS)
 
 
 def oracle_pose(po, opt):
     args = (po["xw"], po["uv"], po["K"], po["rt"], opt)
-    return ref.ba_pose_only(*args) if LOSS is None else robust_ref.ba_pose_only(*args, loss=LOSS)
+    return ref.ba_pose_only(*args) if LOSS is None else oracle_ext.ba_pose_only(*args, loss=LOSS)
 
 
 def outliers(d, key):

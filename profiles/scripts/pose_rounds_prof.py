@@ -3,7 +3,7 @@
     1. one frame, n = 300 / 1000 / 2000, 4 rounds x 10 LM iterations (Huber sqrt(5.991) in rounds
        0-2, octave weights, 20 % gross outliers): device-event time of one rounds call, against four
        sequential lorb_ba_pose_only calls of 10 iterations, and against the C++ reference rounds
-       (tests/rounds_ref.py) on one host core
+       (tests/oracle_ext.py) on one host core
     2. batches of 1 / 64 / 512 / 2048 frames x 1000 observations: frames/s and observation-iterations/s
        (every LM pass visits all observations of its frame, flagged ones are skipped)
     3. lorb_ba_pose_only (n = 2000, 10 iterations) of this build against an older build of the library
@@ -30,7 +30,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
-import rounds_ref as rd  # noqa: E402
+import oracle_ext as rd  # noqa: E402
 from lorb_slam_b200 import capi  # noqa: E402
 from oracle import ref  # noqa: E402
 from test_oracle_pose_rounds_cpu import planted  # noqa: E402
@@ -95,7 +95,7 @@ def single_frame(ctx, reps):
             p_ms.append(event_ms(ctx.stream, four, ctx.sync))
             t = time.perf_counter()
             o = rd.ba_pose_rounds(po["xw"], po["uv"], po["K"], po["rt"], w, opt=fixed_opts(ref),
-                                  loss=(rd.robust_ref.LOSS_HUBER, float(np.sqrt(CHI2))))
+                                  loss=(rd.LOSS_HUBER, float(np.sqrt(CHI2))))
             c_ms.append(1e3 * (time.perf_counter() - t))
         assert o[4] == ROUNDS
         med = lambda v: float(np.median(v))

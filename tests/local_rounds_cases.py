@@ -2,8 +2,8 @@
 share of gross outliers (robust_cases._move), and the mask of the moved observations."""
 import numpy as np
 
+import oracle_ext as rr
 import robust_cases as rc
-import robust_ref as rr
 from lorb_slam_b200 import synth
 
 SCALE_FACTOR = 1.2  # ORB pyramid

@@ -10,8 +10,8 @@ import torch.distributed as dist
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+import oracle_ext as rr  # noqa: E402
 import robust_cases as rc  # noqa: E402
-import robust_ref as rr  # noqa: E402
 from lorb_slam_b200 import capi  # noqa: E402
 
 

@@ -3,7 +3,7 @@ outliers (observations moved 20-80 px), as SearchByProjection mismatches put int
 import numpy as np
 
 from lorb_slam_b200 import synth
-import robust_ref as rr
+import oracle_ext as rr
 
 LOSSES = {"huber": rr.LOSS_HUBER, "softlone": rr.LOSS_SOFTLONE, "cauchy": rr.LOSS_CAUCHY}
 SCALE = 2.0  # pixels: the kernel's knee sits at twice the 1 px observation noise

@@ -1,5 +1,5 @@
 """GPU: local BA with outlier rounds (lorb_ba_local_rounds_batched) against the round reference of
-tests/local_rounds_ref.py on every build path, under all four losses, with and without weights and with
+tests/oracle_ext.py on every build path, under all four losses, with and without weights and with
 fixed observers: cameras and points within 1e-6, the same LM bookkeeping in every round, the same flags
 and counts, chi^2 within 1e-6.  Also: mixed batches, parameters without inliers, the single-round limit,
 a later lorb_ba_local on the same ctx, and refusals."""
@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 import local_rounds_cases as lc
-import local_rounds_ref as lr
+import oracle_ext as lr
 import robust_cases as rc
 from lorb_slam_b200 import capi, synth
 from oracle import ref

@@ -1,5 +1,5 @@
 """GPU: pose-only BA with outlier rounds (lorb_ba_pose_rounds_batched) against the outlier-round
-reference (tests/rounds_ref.py): pose within 1e-6, identical flags, inlier counts, rounds run and LM
+reference (tests/oracle_ext.py): pose within 1e-6, identical flags, inlier counts, rounds run and LM
 trajectories; the single-round limit against lorb_ba_pose_only bit for bit; a mixed batch against the
 single-frame calls bit for bit; refusal of invalid arguments; and the drop-in tracking loop
 (lorb_host::PoseOptimization, then Matcher::SearchByProjection reading its mvbOutlier flags)."""
@@ -8,8 +8,8 @@ import ctypes as C
 import numpy as np
 import pytest
 
+import oracle_ext as rd
 import robust_cases as rc
-import rounds_ref as rd
 from lorb_slam_b200 import capi, synth
 from oracle import ref
 from test_oracle_pose_rounds_cpu import octave_weights, planted

@@ -8,8 +8,8 @@ import sys
 import numpy as np
 import pytest
 
+import oracle_ext as rr
 import robust_cases as rc
-import robust_ref as rr
 from lorb_slam_b200 import capi, synth
 from oracle import ref
 

@@ -1,12 +1,12 @@
-"""CPU: robust losses (Huber, soft-L1, Cauchy) of the BA oracle (tests/robust_ref.py).  The loss functions are checked
+"""CPU: robust losses (Huber, soft-L1, Cauchy) of the BA oracle (tests/oracle_ext.py).  The loss functions are checked
 against finite differences, the trivial loss against the default call bit for bit, and the minimum
 the oracle finds under each loss against scipy.optimize.least_squares, which implements the same
 three losses independently."""
 import numpy as np
 import pytest
 
+import oracle_ext as rr
 import robust_cases as rc
-import robust_ref as rr
 from oracle import ref
 
 TIGHT = dict(max_num_iterations=200, function_tolerance=1e-15, gradient_tolerance=1e-14,

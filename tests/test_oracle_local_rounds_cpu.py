@@ -1,4 +1,4 @@
-"""CPU: the outlier-round reference of lorb_ba_local_rounds_batched (tests/local_rounds_ref.py).  One
+"""CPU: the outlier-round reference of lorb_ba_local_rounds_batched (tests/oracle_ext.py).  One
 round with unit weights and no threshold is the plain and the robust oracle bit for bit; the last round
 is the weighted minimum of scipy.optimize.least_squares on its inlier set; the rounds find planted
 outliers; the depth check flags a point behind its camera; a window without inliers stops at its
@@ -7,9 +7,8 @@ import numpy as np
 import pytest
 
 import local_rounds_cases as lc
-import local_rounds_ref as lr
+import oracle_ext as lr
 import robust_cases as rc
-import robust_ref as rr
 from oracle import ref
 
 TIGHT = dict(max_num_iterations=200, function_tolerance=1e-15, gradient_tolerance=1e-14,
@@ -21,7 +20,7 @@ def test_one_round_without_threshold_is_the_oracle():
     O, F = len(pb["obs_cam"]), pb["F"]
     opt = ref.ba_options(max_num_iterations=10)
     for loss in [None] + [(k, rc.SCALE) for k in rc.LOSSES.values()]:
-        oc, op, o = rr.ba_local(pb, opt, loss=loss)
+        oc, op, o = lr.ba_local(pb, opt, loss=loss)
         for w, fw in ((None, None), (np.ones(O, np.float32), np.ones(F, np.float32))):
             cams, pts, inl, _, finl, _, n_in, sums = lr.ba_local_rounds(
                 pb, w, fw, n_rounds=1, robust_rounds=1, chi2=1e30, opt=opt, loss=loss)

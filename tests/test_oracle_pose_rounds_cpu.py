@@ -1,12 +1,11 @@
-"""CPU: the outlier-round reference of lorb_ba_pose_rounds_batched (tests/rounds_ref.py).  One round
+"""CPU: the outlier-round reference of lorb_ba_pose_rounds_batched (tests/oracle_ext.py).  One round
 without a threshold is the plain and the robust oracle bit for bit; the weighted minimum of the last
 round matches scipy.optimize.least_squares; the rounds find planted outliers; the skip rule holds."""
 import numpy as np
 import pytest
 
+import oracle_ext as rd
 import robust_cases as rc
-import robust_ref as rr
-import rounds_ref as rd
 from oracle import ref
 
 TIGHT = dict(max_num_iterations=200, function_tolerance=1e-15, gradient_tolerance=1e-14,
@@ -45,7 +44,7 @@ def test_one_round_without_threshold_is_the_oracle(weights):
     assert np.array_equal(rt0, rt1) and sums[0] == s0
     assert inl.all() and n_in == 300 and run == 1
     for kind in rc.LOSSES.values():
-        rt0, s0 = rr.ba_pose_only(po["xw"], po["uv"], po["K"], po["rt"], loss=(kind, rc.SCALE))
+        rt0, s0 = rd.ba_pose_only(po["xw"], po["uv"], po["K"], po["rt"], loss=(kind, rc.SCALE))
         rt1, _, _, _, _, sums = rd.ba_pose_rounds(po["xw"], po["uv"], po["K"], po["rt"], w, n_rounds=1,
                                                   robust_rounds=1, chi2=1e30, loss=(kind, rc.SCALE))
         assert np.array_equal(rt0, rt1) and sums[0] == s0
