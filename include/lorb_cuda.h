@@ -686,6 +686,64 @@ int lorb_ba_local_rounds_single(lorb_ctx* ctx, int C, double* cams, int P, doubl
     uint8_t* obs_inlier, double* obs_chi2, uint8_t* fix_inlier, double* fix_chi2,
     int* n_inliers /* [1] */, lorb_ba_summary* summaries /* [n_rounds] or NULL */);
 
+/*
+ * Pose from 2D-3D matches without a prior: batched P3P RANSAC (beyond the reference: the pose half of
+ * VisualOdometry::EstimatePosePnP, and of ORB-SLAM2's per-candidate relocalisation before PoseOptimization).
+ * Problem b owns correspondences [corr_off[b], corr_off[b+1]) of xw / uv / info.  Problems are independent;
+ * no input pose is read.
+ *   corr_off [n_problems+1] int, corr_off[0] = 0, non-decreasing; O = corr_off[n_problems]
+ *   xw [O x 3], uv [O x 2] float    world point and its keypoint
+ *   info [O] float or NULL          per-correspondence weight w (NULL = 1), e.g. 1 / sigma^2 of the octave
+ *   K = {fx, fy, cx, cy} float      shared by every problem
+ *   seeds [n_problems] or NULL      sampler seed of each problem (NULL: the seed of problem b is b)
+ *   out_rt [n_problems x 6] double  (w0, w1, w2, t0, t1, t2): angle-axis R(w) as ba_math.cuh::cam_rotation,
+ *                                   x_c = R(w) X + t, so it feeds lorb_ba_pose_rounds_batched directly
+ *   best_hyp [n_problems]           the selected hypothesis h, or -1
+ *   n_inliers [n_problems]          its inlier count
+ *   out_inlier [O]                  1 = inlier of the selected hypothesis, 0 otherwise
+ *   out_chi2 [O] or NULL            w |r|^2 at the selected hypothesis (+inf behind the camera)
+ * Semantics:
+ * - Camera model: the true pinhole, u = fx x/z + cx, v = fy y/z + cy with (x, y, z) = R(w) X + t.  This is
+ *   not PoseCost's fx-for-v quirk (reference src/bundle_adjust.cpp:51); the two agree when fx = fy.
+ * - Sampler (counter-based): with sm(x) = SplitMix64 (x += 0x9E3779B97F4A7C15;
+ *   z = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9; z = (z ^ (z >> 27)) * 0x94D049BB133111EB; return z ^ (z >> 31)),
+ *   draw k of hypothesis h is r = sm(seed ^ sm(((uint64)h << 8) | k)) and names correspondence
+ *   ((r >> 32) * n) >> 32 of the problem's n.  Draws k = 0, 1, ... that repeat an index already taken are
+ *   skipped until 4 distinct indices are taken; if k passes 255 first, the hypothesis is invalid.  The first
+ *   three indices are the P3P triple, the fourth the check point.
+ * - Hypothesis: a closed-form P3P solve (Lambda Twist, Persson & Nordberg 2018) in fp64 on the triple's
+ *   unit bearings normalise((u - cx) / fx, (v - cy) / fy, 1).  Solutions that put any of the three sample
+ *   points at depth <= 0 are dropped.  Of the rest, the hypothesis is the solution with the smallest squared
+ *   pixel error at the check point, among those that put the check point at depth > 0; ties keep the
+ *   earlier solution in solver order.  A degenerate triple (collinear world points or coincident bearings,
+ *   tolerances in csrc/pnp_math.cuh) has no solution; no solution makes the hypothesis invalid.
+ * - Score: the inlier count, z > 0 and w |r|^2 <= chi2 over all of the problem's correspondences.  The best
+ *   hypothesis has the largest count among the valid ones; ties go to the lowest h.  best_hyp[b] = -1 if the
+ *   problem has fewer than 4 correspondences or no valid hypothesis: then rt is zeros, flags are 0, chi^2
+ *   is +inf and the count is 0.
+ * - out_rt, out_inlier, out_chi2 and n_inliers describe the best hypothesis.  The sampler-to-score arithmetic
+ *   is IEEE correctly rounded (no contraction), so a problem's result depends only on its correspondences,
+ *   its seed and params, and is bit-identical alone or in a batch when seeds are given.
+ * - Refused with LORB_ERR_ARG, before any device work and with every output untouched: bad offsets, a weight
+ *   that is not finite and > 0, fx or fy not finite and > 0, an out-of-range params field, or a NULL
+ *   required pointer (out_inlier may be NULL only when O = 0).
+ * - n_problems = 0 is a no-op.
+ * Two launches on the ctx stream (scoring, then the finalize pass), one upload and one download.
+ */
+typedef struct lorb_pnp_ransac {
+  int n_hypotheses;   /* 300   (1..65536) hypotheses drawn and scored per problem */
+  int reserved;
+  double chi2;        /* 5.991 inlier iff w*|r|^2 <= chi2 (finite, > 0) */
+} lorb_pnp_ransac;
+void lorb_default_pnp_ransac(lorb_pnp_ransac* p);
+
+int lorb_pnp_ransac_batched(lorb_ctx* ctx, int n_problems, const int* corr_off /* [n_problems+1] */,
+    const float* xw /* [O x 3] */, const float* uv /* [O x 2] */, const float* info /* [O] or NULL = 1 */,
+    const float* K /* fx fy cx cy, shared */, const uint64_t* seeds /* [n_problems] or NULL: seed of b = b */,
+    const lorb_pnp_ransac* params,
+    double* out_rt /* [n_problems x 6] */, int* best_hyp /* [n_problems] */, int* n_inliers /* [n_problems] */,
+    uint8_t* out_inlier /* [O] */, double* out_chi2 /* [O] or NULL */);
+
 /* Team size of the library's host-side staging loops (OpenMP) for the calling thread.  Launchers
  * such as torchrun export OMP_NUM_THREADS=1 to every rank; a host that knows how many ranks share
  * the box hands each its share of the cores here.  (omp_set_num_threads on the process's OpenMP

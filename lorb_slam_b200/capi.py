@@ -37,6 +37,7 @@ EXPORTS = [
     "lorb_ba_problem_download", "lorb_ba_problem_destroy", "lorb_ba_set_loss", "lorb_ba_get_loss",
     "lorb_ba_default_pose_rounds", "lorb_ba_pose_rounds_batched",
     "lorb_ba_default_local_rounds", "lorb_ba_local_rounds_batched", "lorb_ba_local_rounds_single",
+    "lorb_default_pnp_ransac", "lorb_pnp_ransac_batched",
     "lorb_dist_get_unique_id",
     "lorb_dist_init", "lorb_dist_finalize", "lorb_dist_allreduce_f64", "lorb_microbench_popc",
     "lorb_microbench_fp64", "lorb_microbench_tensor_i8", "lorb_ctx_profile", "lorb_ctx_profile_read",
@@ -78,6 +79,10 @@ class PoseRounds(C.Structure):
 class LocalRounds(C.Structure):
     _fields_ = [("n_rounds", C.c_int), ("robust_rounds", C.c_int), ("chi2", C.c_double), ("depth_check", C.c_int),
                 ("reserved", C.c_int)]
+
+
+class PnPRansac(C.Structure):
+    _fields_ = [("n_hypotheses", C.c_int), ("reserved", C.c_int), ("chi2", C.c_double)]
 
 
 class FrameView(C.Structure):
@@ -192,6 +197,17 @@ def local_rounds_budgets():
     o = (BAOptions * 2)()
     load_library().lorb_ba_default_local_rounds(None, o)
     return [o[0], o[1]]
+
+
+def pnp_ransac_params(**kw):
+    """lorb_pnp_ransac with its defaults (300 hypotheses, chi2 5.991), fields overridden by kw."""
+    p = PnPRansac()
+    load_library().lorb_default_pnp_ransac(C.byref(p))
+    for k, v in kw.items():
+        if not hasattr(p, k):
+            raise AttributeError(k)
+        setattr(p, k, v)
+    return p
 
 
 def _round_opts(rounds, opt):
@@ -622,6 +638,24 @@ class Context:
         R = rounds.n_rounds
         return (rt, inl.astype(bool), chi2, n_in, run,
                 [[sums[f * R + r].as_dict() for r in range(R)] for f in range(F)])
+
+    def pnp_ransac_batched(self, corr_off, xw, uv, K, info=None, seeds=None, params=None):
+        """lorb_pnp_ransac_batched: problem b owns correspondences corr_off[b]:corr_off[b+1].
+        -> (rt[B,6], best_hyp[B], n_inliers[B], inlier[O] bool, chi2[O])."""
+        co = _arr(corr_off, np.int32).reshape(-1)
+        xw, uv = _arr(xw, np.float32).reshape(-1, 3), _arr(uv, np.float32).reshape(-1, 2)
+        K = _arr(K, np.float32).reshape(4)
+        w = None if info is None else _arr(info, np.float32).reshape(-1)
+        sd = None if seeds is None else _arr(seeds, np.uint64).reshape(-1)
+        params = params or pnp_ransac_params()
+        B, O = len(co) - 1, len(xw)
+        rt = np.zeros((B, 6), np.float64)
+        best, n_in = np.zeros(B, np.int32), np.zeros(B, np.int32)
+        inl, chi2 = np.zeros(O, np.uint8), np.zeros(O, np.float64)
+        _check(self._lib.lorb_pnp_ransac_batched(
+            self._h, B, _ptr(co), _ptr(xw), _ptr(uv), _ptr(w), _ptr(K), _ptr(sd), C.byref(params), _ptr(rt),
+            _ptr(best), _ptr(n_in), _ptr(inl), _ptr(chi2)))
+        return rt, best, n_in, inl.astype(bool), chi2
 
     def ba_local_rounds(self, pb, w=None, fix_w=None, rounds=None, opt=None):
         """lorb_ba_local_rounds_single on one window (the dict of ba_local); w [O] / fix_w [F] weights or None.

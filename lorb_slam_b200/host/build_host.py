@@ -12,7 +12,7 @@ LIBDIR = os.path.join(HERE, "..", "lib")
 OUT = os.path.join(LIBDIR, "libhost_dropin.so")
 SRCS = [os.path.join(HERE, "src", "matcher.cpp"), os.path.join(HERE, "src", "bundle_adjust.cpp"),
         os.path.join(HERE, "src", "ORBextractor.cpp"), os.path.join(HERE, "src", "local_map_index.cpp"),
-        os.path.join(HERE, "src", "pose_optimization.cpp"),
+        os.path.join(HERE, "src", "pose_optimization.cpp"), os.path.join(HERE, "src", "pose_from_matches.cpp"),
         os.path.join(HERE, "test", "harness.cpp")]
 
 

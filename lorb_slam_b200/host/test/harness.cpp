@@ -13,6 +13,7 @@
 #include "../include/matcher.h"
 #include "../include/local_map_index.h"
 #include "../include/pose_optimization.h"
+#include "../include/pose_from_matches.h"
 
 #include <algorithm>
 #include <chrono>
@@ -225,6 +226,42 @@ int harness_pose_rounds_search(int n_kp, const float* x, const float* y, const i
 		else out_state[i] = -1;
 	}
 	return n_in;
+}
+
+// lorb_host::PoseFromMatches on a frame of n keypoints (uv, octaves oct, scale factors sf) whose
+// mvpMapPoints[i] holds a map point at xw[i] iff has_mp[i]; rt (float[6]: R then T) in/out.  Out: which slots
+// still hold their map point, and mvbOutlier.  Returns PoseFromMatches' result.
+int harness_pose_from_matches(int n, const float* xw, const float* uv, const int* oct, const uint8_t* has_mp,
+                              int nlev, const float* sf, const float* K4, int min_inliers, float* rt,
+                              uint8_t* out_has_mp, uint8_t* out_outlier)
+{
+	Camera cam;
+	cam.fx = K4[0]; cam.fy = K4[1]; cam.cx = K4[2]; cam.cy = K4[3];
+	Frame F;
+	F.mpCamera = &cam;
+	F.mnMapPoints = n;
+	F.mvKeysUn.resize(n);
+	F.mvbOutlier.assign(n, false);
+	F.mvScaleFactors.assign(sf, sf+nlev);
+	F.mnScaleLevels = nlev;
+	std::vector<MapPoint> mps(n);
+	F.mvpMapPoints.assign(n, static_cast<MapPoint*>(NULL));
+	for(int i=0;i<n;i++)
+	{
+		F.mvKeysUn[i].pt = cv::Point2f(uv[2*i], uv[2*i+1]);
+		F.mvKeysUn[i].octave = oct[i];
+		mps[i].mWorldPos = cv::Point3f(xw[3*i], xw[3*i+1], xw[3*i+2]);
+		if(has_mp[i]) F.mvpMapPoints[i] = &mps[i];
+	}
+	for(int k=0;k<3;k++) { F.mRvec.at<float>(k) = rt[k]; F.mTvec.at<float>(k) = rt[3+k]; }
+	const int r = lorb_host::PoseFromMatches(&F, min_inliers);
+	for(int k=0;k<3;k++) { rt[k] = F.mRvec.at<float>(k); rt[3+k] = F.mTvec.at<float>(k); }
+	for(int i=0;i<n;i++)
+	{
+		out_has_mp[i] = F.mvpMapPoints[i] ? 1 : 0;
+		out_outlier[i] = F.mvbOutlier[i] ? 1 : 0;
+	}
+	return r;
 }
 
 // BA::ProjectPoseOptimization: rt (float[6]: R then T) in/out

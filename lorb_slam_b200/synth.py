@@ -354,6 +354,50 @@ def make_pose_only(seed=0, n=500, pixel_noise=1.0, pose_noise=(0.02, 0.1)):
     return dict(n=n, xw=xw, uv=uv, K=K.copy(), rt=rt0, rt_true=np.concatenate([rv, tv]))
 
 
+def make_pnp_problems(seed=0, n=300, n_problems=1, outlier_frac=0.3, pixel_noise=1.0, K=None, n_levels=8,
+                      scale=1.2, collinear=False, noise="gauss"):
+    """Inputs of lorb_pnp_ransac_batched: n_problems independent 2D-3D match sets of n correspondences each
+    (n an int or a sequence of n_problems ints), each with its own planted pose (rt_true [B, 6], angle-axis +
+    translation, x_c = R X + t).  Points lie 3-20 m in front of the camera; keypoints get Gaussian noise of
+    pixel_noise * scale^octave (octaves drawn as an ORB pyramid fills them), so info = 1 / sigma^2 of the octave
+    are the true inverse variances (noise="uniform": uniform in +-pixel_noise * scale^octave per axis instead);
+    `outlier_frac` of the keypoints are replaced by uniform pixels (mismatches).  collinear=True puts every world
+    point of a problem on one line."""
+    rng = np.random.default_rng(seed + 7919)
+    K = K_DEFAULT if K is None else np.asarray(K, np.float32)
+    sizes = [int(n)] * n_problems if np.isscalar(n) else [int(v) for v in n]
+    wl = (1.0 / scale) ** np.arange(n_levels)
+    xw, uv, info, outl, rts = [], [], [], [], []
+    for m in sizes:
+        rv = rng.normal(0, 0.5, 3)
+        tv = rng.normal(0, 1.0, 3)
+        if collinear:
+            a, d = rng.normal(0, 1, 3) + [0, 0, 10], rng.normal(0, 1, 3)
+            Xc = a + np.outer(rng.uniform(-3, 3, m), d / np.linalg.norm(d))
+        else:
+            Xc = np.stack([rng.uniform(-4, 4, m), rng.uniform(-3, 3, m), rng.uniform(3, 20, m)], 1)
+        R = rodrigues(rv)
+        X = (Xc - tv) @ R  # R^T (Xc - t)
+        oc = rng.choice(n_levels, size=m, p=wl / wl.sum())
+        sig = pixel_noise * scale ** oc
+        nz = rng.normal(0, 1, (m, 2)) if noise == "gauss" else rng.uniform(-1, 1, (m, 2))
+        u = K[0] * Xc[:, 0] / Xc[:, 2] + K[2] + nz[:, 0] * sig
+        v = K[1] * Xc[:, 1] / Xc[:, 2] + K[3] + nz[:, 1] * sig
+        bad = rng.random(m) < outlier_frac
+        u[bad] = rng.uniform(0, 2 * K[2], bad.sum())
+        v[bad] = rng.uniform(0, 2 * K[3], bad.sum())
+        xw.append(X)
+        uv.append(np.stack([u, v], 1))
+        info.append(1.0 / (scale ** oc) ** 2)
+        outl.append(bad)
+        rts.append(np.concatenate([rv, tv]))
+    cat = lambda a, d: np.ascontiguousarray(np.concatenate(a).reshape(-1, d)) if a else np.zeros((0, d))
+    return dict(corr_off=np.concatenate([[0], np.cumsum(sizes)]).astype(np.int32), K=K.copy(),
+                xw=cat(xw, 3).astype(np.float32), uv=cat(uv, 2).astype(np.float32),
+                info=cat(info, 1).reshape(-1).astype(np.float32), outlier=cat(outl, 1).reshape(-1).astype(bool),
+                rt_true=np.array(rts).reshape(-1, 6))
+
+
 def batch_windows(pbs):
     """Concatenate independent windows into the offset-array form of
     lorb_ba_local_batched (observation indices stay window-local)."""
